@@ -2,7 +2,7 @@
 """bench.py -- 48 kHz audio-seconds enhanced per wall-second (batched enhance()), BASELINE.json's
 metric, on N GPUs of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2..5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2..5] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the whole enhancement path (pad -> STFT -> features -> DNN -> mask + deep
@@ -23,6 +23,10 @@ parity; `--config N` makes one of them the headline instead.
             steps; `traffic` from the ncu capture committed under profiles/ (same batch)
   parity  : RMS of 4 streams of the timed batch's output against the CPU oracle (outside the timed region)
   cpu_baseline: the CPU oracle port (C DSP + torch-CPU DNN) on this box's host cores, bounded sample
+
+--dump-outputs DIR writes the headline's enhanced audio of the last timed step to DIR/enhanced.npy (float32
+[streams, samples]): a fixed, seeded sample of the batch's streams (all of them when they fit DUMP_BYTES), so that two
+builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,6 +39,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True   # the tree may be read-only; nothing is written into it
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
@@ -53,6 +58,7 @@ BASELINE_NAME = {2: "BASELINE.json configs[1]", 3: "BASELINE.json configs[2]", 4
 FLOP_PER_FRAME = {"DeepFilterNet3": 6_614_784, "DeepFilterNet2": 6_956_800, "DeepFilterNet3_ll": 21_846_784}
 DTYPE = "f32 (bf16x3 tensor-core contractions, fp32 accumulate; DSP and gates IEEE fp32)"
 PARITY_TOL = 1e-4  # BASELINE.json north_star: RMS vs the reference path
+DUMP_BYTES = 48 << 20  # --dump-outputs budget
 
 
 def kernel_model(cfg, g: dict) -> dict:
@@ -310,6 +316,17 @@ def cpu_reference_run(cfg, sd, seconds: int, steps: int, warmup: int, threads: i
     return streams * seconds * steps / dt, dt / steps, streams
 
 
+def dump_sample(out):
+    """A fixed, seeded sample of the streams of `out` [streams, T] (and a prefix of each when one stream alone exceeds
+    DUMP_BYTES), copied to the host as float32."""
+    import torch
+    streams, T = out.shape
+    cols = min(T, DUMP_BYTES // 4)
+    k = max(1, min(streams, DUMP_BYTES // (4 * cols)))
+    rows = torch.randperm(streams, generator=torch.Generator().manual_seed(0))[:k].sort().values
+    return out[rows.to(out.device), :cols].float().cpu()
+
+
 def ctypes_buf():
     import ctypes
     return ctypes.create_string_buffer(1 << 16)
@@ -353,7 +370,7 @@ class Ctx:
 
 
 def measure(ctx: Ctx, cfg_id: int, model_name: str, streams: int, seconds: int, steps: int, warmup: int,
-            roofline_kernel=None, parity_streams: int = 4, clocks=None):
+            roofline_kernel=None, parity_streams: int = 4, clocks=None, dump: bool = False):
     """One workload on this process' GPU (all ranks run it in lock step): returns the JSON fields."""
     import torch
     from deepfilternet_b200 import DfNet, _lib, enhance, enhance_device, libdf
@@ -388,6 +405,7 @@ def measure(ctx: Ctx, cfg_id: int, model_name: str, streams: int, seconds: int, 
     ctx.sync_all()
     ms = ev0.elapsed_time(ev1)
     launches = int(L.dfb_kernel_launches() - launches0)
+    dumped = dump_sample(out) if dump else None   # the last timed step's output, before later passes reuse `out`
     # ---------------- end to end through the public API with host buffers
     for _ in range(2):
         enhance(model, st, host_in, out=host_out)
@@ -483,6 +501,8 @@ def measure(ctx: Ctx, cfg_id: int, model_name: str, streams: int, seconds: int, 
            "e2e": {"value": e2e, "unit": "audio-s/s", "h2d_bytes_per_step": int(host_in.numel() * 4),
                    "d2h_bytes_per_step": int(host_out.numel() * 4), "ms_per_step": t_e2e * 1e3 / steps},
            "roofline": roofline, "per_gpu": per_gpu, "parity": parity, "workspace_bytes": model.workspace_bytes()}
+    if dumped is not None:
+        res["dumped"] = dumped
     # RTF at batch = 1 (BASELINE.json metric, second half): one stream, device resident and end to end
     a1 = audio[:1].contiguous()
     o1 = torch.empty_like(a1)
@@ -520,7 +540,11 @@ def main():
     ap.add_argument("--extra", default=None, help="comma list of extra configs (default: 3,4,5,6 at N=1; 4 at N=4; 5 at N=8; 'none')")
     ap.add_argument("--roofline-kernel", default=None, help="kernel to report (default: the one with most time)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the headline's output of the last timed step (a fixed, seeded sample of streams) as DIR/enhanced.npy")
     a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     n_gpus = a.gpus
     a.warmup = max(a.warmup, 3) if a.impl == "ours" else a.warmup
@@ -558,8 +582,13 @@ def main():
     ctx = Ctx(a)
     clocks = ClockSampler(ctx.dev)
     clocks.start()
-    head, cfg, sd = measure(ctx, cfg_id, model_name, streams, seconds, a.steps, a.warmup, a.roofline_kernel, clocks=clocks)
+    head, cfg, sd = measure(ctx, cfg_id, model_name, streams, seconds, a.steps, a.warmup, a.roofline_kernel, clocks=clocks,
+                            dump=bool(a.dump_outputs) and ctx.rank == 0)
     clk = clocks.stop()
+    if "dumped" in head:
+        import numpy as np
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        np.save(os.path.join(a.dump_outputs, "enhanced.npy"), head.pop("dumped").numpy())
     if a.extra is None:
         extra_ids = {1: [3, 4, 5, 6], 4: [4], 8: [5]}.get(n_gpus, [])
         extra_ids = [i for i in extra_ids if i != cfg_id] if cfg_id == 2 else []

@@ -1,13 +1,13 @@
 """Generate the committed golden fixtures under tests/golden/ by running the REFERENCE's own
-Python modules (imported from /root/reference, which only exists in the build container) on top
-of the CPU oracle for the Rust DSP.  Run:  python oracle/gen_golden.py
+Python modules (imported from $DFB_REFERENCE_ROOT) on top of the CPU oracle for the Rust DSP.
+The models carry the seeded random weights of oracle/random_models.py (the shipped checkpoints are
+too large to keep in the repository).  Run:  DFB_REFERENCE_ROOT=<reference tree> python oracle/gen_golden.py
 
 Outputs (small; committed):
   tests/golden/erb_widths.json       ERB band widths recovered from the `erb_fb` buffers stored in
                                      the shipped checkpoints (pins libDF/src/lib.rs:68-100 bit-exact)
-  tests/golden/kat.json              SI-SDR known answers of df/scripts/test_df.py:44-78 and the
-                                     values the reference modules + oracle produce here
-  tests/golden/dfnet_<model>.npz     reference DfNet.forward / enhance() outputs on a 0.5 s excerpt
+  tests/golden/kat.json              SI-SDR of the reference modules + oracle on the whole recording
+  tests/golden/dfnet_<model>.npz     reference DfNet.forward / enhance() outputs on a 0.2 s excerpt
   tests/golden/assets/*.wav          the two 48 kHz test recordings used by the reference's KAT
 """
 from __future__ import annotations
@@ -16,6 +16,7 @@ import json
 import os
 import shutil
 import sys
+import tempfile
 
 import numpy as np
 import torch
@@ -23,14 +24,15 @@ import torch
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 sys.path.insert(0, HERE)
+import random_models  # noqa: E402
 import ref_harness as rh  # noqa: E402
 
 GOLD = os.path.join(ROOT, "tests", "golden")
-TARGETS = {  # DeepFilterNet/df/scripts/test_df.py:44-78
-    "DeepFilterNet": 18.88543128967285,
-    "DeepFilterNet2": 19.41733717918396,
-    "DeepFilterNet3": 20.014915466308594,
-}
+
+
+def excerpt(noisy: torch.Tensor) -> torch.Tensor:
+    """0.2 s, two channels (second = time-shifted, attenuated) to exercise batching."""
+    return torch.stack([noisy[0, 96000:105600], 0.5 * noisy[0, 130000:139600]])
 
 
 def main():
@@ -42,63 +44,40 @@ def main():
     from df.enhance import df_features, enhance, init_df
     import torch.nn.functional as F
 
+    widths = {}
+    for name in ("DeepFilterNet3", "DeepFilterNet2"):
+        fb = init_df(os.path.join(d, name), log_file=None, log_level="ERROR")[0].state_dict()["erb_fb"].numpy()
+        # [F, E], non-zero pattern = band membership
+        widths[name] = [int((fb[:, b] != 0).sum()) for b in range(fb.shape[1])]
+        # bands must be contiguous and ordered
+        starts = [int(np.argmax(fb[:, b] != 0)) for b in range(fb.shape[1])]
+        assert starts == list(np.cumsum([0] + widths[name][:-1]))
+
     noisy = torch.from_numpy(rh.read_wav(os.path.join(GOLD, "assets", "noisy_snr0.wav")))
     clean = rh.read_wav(os.path.join(GOLD, "assets", "clean_freesound_33711.wav"))
-    widths, kat = {}, {}
-    for name in ("DeepFilterNet3", "DeepFilterNet2", "DeepFilterNet"):
-        model, st, _, epoch = init_df(os.path.join(d, name), log_file=None, log_level="ERROR")
-        sd = model.state_dict()
-        if "erb_fb" in sd:
-            fb = sd["erb_fb"].numpy()  # [F, E], non-zero pattern = band membership
-            widths[name] = [int((fb[:, b] != 0).sum()) for b in range(fb.shape[1])]
-            # bands must be contiguous and ordered
-            starts = [int(np.argmax(fb[:, b] != 0)) for b in range(fb.shape[1])]
-            assert starts == list(np.cumsum([0] + widths[name][:-1]))
+    kat = {}
+    tmp = tempfile.mkdtemp()
+    for name in ("DeepFilterNet3", "DeepFilterNet2", "DeepFilterNet", "DeepFilterNet3_ll"):
+        model, st, _ = rh.init_random_df(tmp, name)
         out = enhance(model, st, noisy, pad=True)
-        kat[name] = dict(target=TARGETS[name], reference_modules_plus_oracle=rh.si_sdr(clean, out.numpy()),
-                         epoch=int(epoch), n_samples=int(noisy.shape[1]))
+        kat[name] = dict(target=rh.si_sdr(clean, out.numpy()), epoch=random_models.epoch(name), n_samples=int(noisy.shape[1]))
         print(name, kat[name])
         if name == "DeepFilterNet":
-            continue  # DFN1 is a "next" row (SURVEY.md 8f); only its KAT value is recorded
-        # short excerpt, two channels (second = time-shifted, attenuated) to exercise batching
-        x = torch.stack([noisy[0, 96000:120000], 0.5 * noisy[0, 130000:154000]])
+            continue  # oracle/gen_golden_v1.py
+        x = excerpt(noisy)
         y = enhance(model, st, x, pad=True)
-        y_nopad = enhance(model, st, x, pad=False)
-        y_att = enhance(model, st, x, pad=True, atten_lim_db=12.0)
         xa = F.pad(x, (0, st.fft_size()))
         spec, ef, sf = df_features(xa, st, 96)
         with torch.no_grad():
             spec_e, m, lsnr, c = model(spec.clone(), ef, sf)
-        np.savez_compressed(
-            os.path.join(GOLD, f"dfnet_{name}.npz"), audio=x.numpy(), enhanced=y.numpy(),
-            enhanced_nopad=y_nopad.numpy(), enhanced_atten12=y_att.numpy(),
-            spec=spec.numpy(), feat_erb=ef.numpy(), feat_spec=sf.numpy(), spec_e=spec_e.numpy(),
-            m=m.numpy(), lsnr=lsnr.numpy(),
-            coefs=(c if c.dim() == 5 else torch.zeros(0)).numpy())
-    # DeepFilterNet3_ll ships only as ONNX: build the reference DfNet from its config (epoch="none"),
-    # load the transplanted weights (deepfilternet_b200/onnx_import.py) and record the reference outputs.
-    sys.path.insert(0, ROOT)
-    from deepfilternet_b200.config import load_config
-    from deepfilternet_b200.onnx_import import state_dict_from_onnx_dir
-    ll_dir = os.path.join(d, "DeepFilterNet3_ll_onnx")
-    model, st, _, _ = init_df(ll_dir, log_file=None, log_level="ERROR", epoch="none")
-    sd_ll = state_dict_from_onnx_dir(ll_dir, load_config(os.path.join(ll_dir, "config.ini"), env={}))
-    missing, unexpected = model.load_state_dict(sd_ll, strict=False)
-    assert not unexpected and all(k in ("erb_fb", "mask.erb_inv_fb") or "df_fc_a" in k for k in missing), (missing, unexpected)
-    model.eval()
-    out = enhance(model, st, noisy, pad=True)
-    kat["DeepFilterNet3_ll"] = dict(target=None, reference_modules_plus_oracle=rh.si_sdr(clean, out.numpy()), epoch=0,
-                                    n_samples=int(noisy.shape[1]))
-    print("DeepFilterNet3_ll", kat["DeepFilterNet3_ll"])
-    x = torch.stack([noisy[0, 96000:120000], 0.5 * noisy[0, 130000:154000]])
-    y = enhance(model, st, x, pad=True)
-    xa = F.pad(x, (0, st.fft_size()))
-    spec, ef, sf = df_features(xa, st, 96)
-    with torch.no_grad():
-        spec_e, m, lsnr, c = model(spec.clone(), ef, sf)
-    np.savez_compressed(os.path.join(GOLD, "dfnet_DeepFilterNet3_ll.npz"), audio=x.numpy(), enhanced=y.numpy(),
-                        spec=spec.numpy(), feat_erb=ef.numpy(), feat_spec=sf.numpy(), spec_e=spec_e.numpy(), m=m.numpy(),
-                        lsnr=lsnr.numpy())
+        arrays = dict(audio=x.numpy(), enhanced=y.numpy(), spec=spec.numpy(), feat_erb=ef.numpy(), feat_spec=sf.numpy(),
+                      spec_e=spec_e.numpy(), m=m.numpy(), lsnr=lsnr.numpy())
+        if name != "DeepFilterNet3_ll":
+            arrays.update(enhanced_nopad=enhance(model, st, x, pad=False).numpy(),
+                          enhanced_atten12=enhance(model, st, x, pad=True, atten_lim_db=12.0).numpy(),
+                          coefs=(c if c.dim() == 5 else torch.zeros(0)).numpy())
+        np.savez_compressed(os.path.join(GOLD, f"dfnet_{name}.npz"), **arrays)
+    shutil.rmtree(tmp)
     with open(os.path.join(GOLD, "erb_widths.json"), "w") as f:
         json.dump(dict(params=dict(sr=48000, fft_size=960, nb_bands=32, min_nb_freqs=2),
                        from_checkpoint_erb_fb=widths), f, indent=1)

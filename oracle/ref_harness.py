@@ -1,9 +1,9 @@
-"""Import the reference's *Python* package (``/root/reference/DeepFilterNet/df``) in this
-container with the CPU oracle bound as module ``libdf``.
+"""Import the reference's *Python* package (``$DFB_REFERENCE_ROOT/DeepFilterNet/df``) with the
+CPU oracle bound as module ``libdf``.
 
-TEST INFRASTRUCTURE ONLY.  Used by oracle/gen_golden.py (fixture generation) and by tests that
-skip when /root/reference is absent (it does not exist on the GPU box).  Recipe from
-SURVEY.md Appendix C:
+TEST INFRASTRUCTURE ONLY.  Used by oracle/gen_golden*.py (fixture generation) and, for
+``read_wav`` / ``si_sdr``, by the tests.  The reference tree is found at $DFB_REFERENCE_ROOT.
+Recipe from SURVEY.md Appendix C:
   * the reference's Rust ``libdf`` cannot be built here, so ``sys.modules['libdf']`` is the
     oracle binding (oracle/libdf_oracle.py);
   * torchaudio 2.11 dropped ``AudioMetaData`` which ``df/io.py:10-19`` needs at import time;
@@ -17,14 +17,15 @@ import glob
 import os
 import sys
 import tarfile
+import tempfile
 import types
 import wave
 import zipfile
 
 import numpy as np
 
-REF_ROOT = os.environ.get("DFB_REFERENCE_ROOT", "/root/reference")
-SCRATCH = os.environ.get("DFB_REF_SCRATCH", "/tmp/dfb_ref_models")
+REF_ROOT = os.environ.get("DFB_REFERENCE_ROOT", "")
+SCRATCH = os.environ.get("DFB_REF_SCRATCH", os.path.join(tempfile.gettempdir(), "dfb_ref_models"))
 
 
 def available() -> bool:
@@ -80,6 +81,20 @@ def import_reference():
     import df.enhance  # noqa: F401
 
     return df
+
+
+def init_random_df(root: str, name: str, **kw):
+    """The reference's ``init_df`` on the random-weight model directory of ``random_models`` (written under `root`):
+    the reference builds the model from the shipped config, then loads the seeded weights; the only tensors it keeps
+    from its own init are the ERB filterbanks, which it computes from the DF state."""
+    import random_models
+    d = random_models.write_model_dir(root, name)
+    from df.enhance import init_df
+    model, st, suffix, _ = init_df(d, log_file=None, log_level="ERROR", epoch="none", **kw)
+    missing, unexpected = model.load_state_dict(random_models.state_dict(name), strict=False)
+    assert not unexpected and set(missing) <= {"erb_fb", "mask.erb_inv_fb"}, (missing, unexpected)
+    model.eval()
+    return model, st, suffix
 
 
 def read_wav(path: str) -> np.ndarray:

@@ -9,7 +9,6 @@ for p in (ROOT, os.path.join(ROOT, "oracle")):
         sys.path.insert(0, p)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-MODEL_DIR = os.path.join(ROOT, "models", "_ref")
 
 
 def pytest_configure(config):
@@ -22,14 +21,11 @@ def golden_dir():
 
 
 @pytest.fixture(scope="session")
-def model_dir():
-    """models/_ref is unpacked from the reference archives by __graft_entry__.build()."""
-    if not os.path.isdir(os.path.join(MODEL_DIR, "DeepFilterNet3")):
-        try:
-            import __graft_entry__ as g
-            g._unpack_reference_models()
-        except Exception:
-            pass
-    if not os.path.isdir(os.path.join(MODEL_DIR, "DeepFilterNet3")):
-        pytest.skip("pretrained weights not unpacked (models/_ref); run __graft_entry__.build() where /root/reference exists")
-    return MODEL_DIR
+def model_dir(tmp_path_factory):
+    """Model directories laid out like the shipped ones (config.ini + checkpoints/): the shipped configs with seeded
+    random weights (oracle/random_models.py), the weights the golden fixtures were made with."""
+    import random_models
+    root = str(tmp_path_factory.mktemp("models"))
+    for name in random_models.CHECKPOINTS:
+        random_models.write_model_dir(root, name)
+    return root

@@ -199,9 +199,9 @@ def test_golden_reference_outputs(name, golden_dir, model_dir):
     assert rms(spec_e, g["spec_e"]) < TOL_SPEC and rms(m, g["m"]) < TOL_M and np.abs(lsnr.numpy() - g["lsnr"]).max() < TOL_LSNR
 
 
-def test_ll_onnx_model_end_to_end(golden_dir, model_dir):
-    """DeepFilterNet3_ll (ONNX-only weights, H = 512, zero look-ahead, kt = 2 convs): init_df on the ONNX
-    directory, against the reference modules' outputs with the transplanted weights."""
+def test_ll_model_end_to_end(golden_dir, model_dir):
+    """DeepFilterNet3_ll (H = 512, zero look-ahead, kt = 2 convs): init_df on its model directory, against the
+    reference modules' outputs with the same weights."""
     g = np.load(os.path.join(golden_dir, "dfnet_DeepFilterNet3_ll.npz"))
     model, st, suffix, epoch = init_df(os.path.join(model_dir, "DeepFilterNet3_ll"), log_level="ERROR")
     assert (model.cfg.conv_lookahead, model.cfg.df_lookahead, model.cfg.emb_hidden_dim) == (0, 0, 512)
@@ -212,7 +212,8 @@ def test_ll_onnx_model_end_to_end(golden_dir, model_dir):
 
 @pytest.mark.parametrize("name", ["DeepFilterNet3", "DeepFilterNet2"])
 def test_si_sdr_known_answer_gpu(name, golden_dir, model_dir):
-    """The reference CI's known answer (df/scripts/test_df.py:44-78, atol = rtol = 1e-4) on the CUDA path."""
+    """The reference CI's known answer check (df/scripts/test_df.py:44-78, atol = rtol = 1e-4) on the CUDA path, against
+    the reference modules' value for the weights of model_dir."""
     import ref_harness as rh
     kat = json.load(open(os.path.join(golden_dir, "kat.json")))[name]
     model, st, _, epoch = init_df(os.path.join(model_dir, name), log_level="ERROR")
@@ -314,15 +315,12 @@ def test_wide_batch_matches_oracle(states):
 
 
 # ------------------------------------------------------------------ BASELINE configs at size ----
-def _pretrained_or_random(name, kind, model_dir_path):
-    """(cfg, state_dict) of a shipped model when models/_ref travelled with the snapshot, else random weights."""
+def _model_dir_weights(name, model_dir_path):
+    """(cfg, state_dict) of a model directory laid out like the shipped ones."""
     p = os.path.join(model_dir_path, name)
-    if os.path.isdir(os.path.join(p, "checkpoints")):
-        cfg = load_config(os.path.join(p, "config.ini"), env={})
-        cp, _ = find_checkpoint(os.path.join(p, "checkpoints"))
-        return cfg, load_state_dict_file(cp)
-    cfg = cfg_of(kind)
-    return cfg, random_state_dict(cfg, seed=3)
+    cfg = load_config(os.path.join(p, "config.ini"), env={})
+    cp, _ = find_checkpoint(os.path.join(p, "checkpoints"))
+    return cfg, load_state_dict_file(cp)
 
 
 @pytest.mark.parametrize("name,kind,B,seconds,rows", [
@@ -339,7 +337,7 @@ def test_baseline_configs_at_size(states, model_dir, name, kind, B, seconds, row
         cfg = cfg_of("ll")
         sd = random_state_dict(cfg, seed=3)
     else:
-        cfg, sd = _pretrained_or_random(name, kind, model_dir)
+        cfg, sd = _model_dir_weights(name, model_dir)
     model = DfNet(cfg, sd, st)
     audio = synth_audio(B, 48000 * seconds, seed=77, device="cuda")
     out = enhance_device(model, st, audio)
@@ -377,7 +375,7 @@ def test_stream_groups_with_ragged_last_group(states):
 
 @pytest.mark.parametrize("name", ["DeepFilterNet3", "DeepFilterNet2"])
 def test_whole_asset_rms_against_oracle(name, golden_dir, model_dir):
-    """Pretrained weights on the whole 10.6 s reference recording: RMS(out - oracle) <= 1e-4 (the SI-SDR KAT above
+    """The whole 10.6 s reference recording: RMS(out - oracle) <= 1e-4 (the SI-SDR KAT above
     is a scalar with 1e-4 relative slack; this compares every sample)."""
     import ref_harness as rh
     model, st, _, _ = init_df(os.path.join(model_dir, name), log_level="ERROR")
@@ -609,7 +607,7 @@ def test_v1_golden_reference_outputs(golden_dir, model_dir):
 
 
 def test_v1_si_sdr_known_answer_and_whole_asset(golden_dir, model_dir):
-    """The third known answer of the reference CI (df/scripts/test_df.py:45-55: DeepFilterNet 18.885 dB) on the CUDA path, and
+    """The third known answer check of the reference CI (df/scripts/test_df.py:45-55: DeepFilterNet) on the CUDA path, and
     every sample of the 10.6 s recording against the oracle."""
     import dfnet1_oracle as O1
     import ref_harness as rh

@@ -81,7 +81,7 @@ def test_unit_norm_matches_exponential_unit_norm():
 
 @pytest.mark.parametrize("name", ["DeepFilterNet3", "DeepFilterNet2"])
 def test_dfnet_oracle_matches_reference_modules(name, golden_dir, model_dir):
-    """tests/golden/dfnet_<model>.npz were produced by the reference's own DfNet / enhance()."""
+    """tests/golden/dfnet_<model>.npz were produced by the reference's own DfNet / enhance() with the same weights."""
     g = np.load(os.path.join(golden_dir, f"dfnet_{name}.npz"))
     cfg = load_config(os.path.join(model_dir, name, "config.ini"), env={})
     sd = load_state_dict_file(find_checkpoint(os.path.join(model_dir, name, "checkpoints"))[0])
@@ -101,13 +101,12 @@ def test_dfnet_oracle_matches_reference_modules(name, golden_dir, model_dir):
     assert float(np.sqrt(((o3.numpy() - g["enhanced_atten12"]) ** 2).mean())) < 1e-6
 
 
-def test_ll_oracle_matches_reference_modules_with_transplanted_onnx_weights(golden_dir, model_dir):
-    """DeepFilterNet3_ll ships only as ONNX: tests/golden/dfnet_DeepFilterNet3_ll.npz holds the outputs of the
-    reference DfNet (built from the _ll config) carrying the transplanted weights."""
-    from deepfilternet_b200.onnx_import import state_dict_from_onnx_dir
+def test_ll_oracle_matches_reference_modules(golden_dir, model_dir):
+    """tests/golden/dfnet_DeepFilterNet3_ll.npz holds the outputs of the reference DfNet built from the _ll config
+    (H = 512, zero look-ahead, kt = 2 convs)."""
     d = os.path.join(model_dir, "DeepFilterNet3_ll")
     cfg = load_config(os.path.join(d, "config.ini"), env={})
-    sd = state_dict_from_onnx_dir(d, cfg)
+    sd = load_state_dict_file(find_checkpoint(os.path.join(d, "checkpoints"))[0])
     g = np.load(os.path.join(golden_dir, "dfnet_DeepFilterNet3_ll.npz"))
     out, aux = O.enhance(sd, cfg.as_dict(), torch.from_numpy(g["audio"]), pad=True, return_all=True)
     assert np.abs(aux["m"].numpy() - g["m"]).max() < 1e-5
@@ -115,33 +114,10 @@ def test_ll_oracle_matches_reference_modules_with_transplanted_onnx_weights(gold
     assert float(np.sqrt(((out.numpy() - g["enhanced"]) ** 2).mean())) < 1e-6
 
 
-def test_onnx_transplant_equals_checkpoint(model_dir):
-    """The ONNX export of DeepFilterNet3 ships next to its checkpoint: the transplant must reproduce the
-    checkpoint's packed tensors (BN folded by torch at export vs folded here)."""
-    from deepfilternet_b200.onnx_import import state_dict_from_onnx_dir
-    from deepfilternet_b200.weights import pack_state_dict
-    d = os.path.join(model_dir, "DeepFilterNet3_onnx")
-    if not os.path.isdir(d):
-        pytest.skip("DeepFilterNet3_onnx not unpacked")
-    cfg = load_config(os.path.join(model_dir, "DeepFilterNet3", "config.ini"), env={})
-    pa, da = pack_state_dict(state_dict_from_onnx_dir(d, cfg), cfg)
-    pb, db = pack_state_dict(load_state_dict_file(find_checkpoint(os.path.join(model_dir, "DeepFilterNet3", "checkpoints"))[0]), cfg)
-    assert da == db and set(pb) <= set(pa)
-    def value(k, a):
-        if k.endswith(".pw_sw"):  # packed BF16 hi | lo planes: compare the numbers they represent
-            bf = torch.from_numpy(a.view(np.int16).copy()).view(torch.bfloat16).to(torch.float32).numpy()
-            return bf[: bf.size // 2] + bf[bf.size // 2:]
-        return a
-
-    for k, b in pb.items():
-        a, b = value(k, pa[k]), value(k, b)
-        rel = 2.0 ** -15 if k.endswith(".pw_sw") else 1e-6  # hi + lo carries 16 mantissa bits
-        assert np.abs(a - b).max() <= rel * (np.abs(b).max() + 1e-12) + 1e-9, k
-
-
 @pytest.mark.parametrize("name", ["DeepFilterNet3", "DeepFilterNet2"])
 def test_si_sdr_known_answer(name, golden_dir, model_dir):
-    """DeepFilterNet/df/scripts/test_df.py:44-78: SI-SDR of enhance(noisy_snr0) vs clean, atol=rtol=1e-4."""
+    """DeepFilterNet/df/scripts/test_df.py:44-78 on the weights of model_dir: SI-SDR of enhance(noisy_snr0) vs clean against
+    the reference modules' value (tests/golden/kat.json), atol=rtol=1e-4."""
     import ref_harness as rh
     kat = json.load(open(os.path.join(golden_dir, "kat.json")))[name]
     cfg = load_config(os.path.join(model_dir, name, "config.ini"), env={})
@@ -229,7 +205,7 @@ def test_v1_oracle_matches_reference_modules(golden_dir, model_dir):
 
 
 def test_v1_si_sdr_known_answer(golden_dir, model_dir):
-    """df/scripts/test_df.py:45-55: DeepFilterNet (v1) 18.88543128967285 dB, atol = rtol = 1e-4."""
+    """df/scripts/test_df.py:45-55 for DeepFilterNet (v1) on the weights of model_dir, atol = rtol = 1e-4."""
     import dfnet1_oracle as O1
     import ref_harness as rh
     kat = json.load(open(os.path.join(golden_dir, "kat.json")))["DeepFilterNet"]
