@@ -106,12 +106,14 @@ struct Arena {
 
 constexpr int kMaxErb = 64;
 
-// Device-resident tables of one DSP state (fft 960 / hop 480 kernels).
+// Device-resident tables of one DSP state.  M = fft / 2; the 960 / 480 kernels read tw_a_*, every other geometry the
+// runtime FFT (dfb_fft.cuh) with tw_m.
 struct DspTables {
     const float *window;     // [fft]
-    const float2 *tw_a_fwd;  // [24][20]  w480^{-lane k1}
+    const float2 *tw_a_fwd;  // [24][20]  w480^{-lane k1} (fft 960 only, else null)
     const float2 *tw_a_inv;  // [24][20]  conj
-    const float2 *tw960;     // [241]     e^{-2 pi i k / 960}
+    const float2 *tw_split;  // [M/2 + 1] e^{-2 pi i k / fft}  (real split / merge steps)
+    const float2 *tw_m;      // [M]       e^{-2 pi i k / M}    (runtime FFT passes)
     const int *erb_off;      // [E + 1]
     const float *erb_kinv;   // [E]  1 / width
     const unsigned char *band_of_bin;  // [F]
@@ -152,8 +154,8 @@ struct ApplyParams {
     float atten_lim;      // 0 = off
     // carried ISTFT state (pyDF synthesis(reset=False), mode 0 only): channel 0 starts from init_tail,
     // channel c > 0 from the tail left by channel c - 1; the tail after the last frame goes to final_tail
-    const float *init_tail;  // [hop] or null
-    float *final_tail;       // [hop] or null
+    const float *init_tail;  // [fft - hop] or null
+    float *final_tail;       // [fft - hop] or null
     int carry;
 };
 
@@ -162,7 +164,8 @@ struct ApplyParams {
 struct dfb_state;
 namespace dfb {
 // frame window of launch_analysis: frames [t_begin, t_begin + nf) of a signal of T samples per row (row pitch row_stride,
-// 0 = T) go to rows out_t0 ... of buffers holding Tbuf frames per stream
+// 0 = T) go to rows out_t0 ... of buffers holding Tbuf frames per stream.  Frame t covers samples
+// [t hop - (fft - hop), t hop + hop); samples before 0 come from d_init_mem [C][fft - hop] (null: zeros).
 struct AnaWindow { int t_begin, nf, out_t0, Tbuf; int64_t row_stride; };
 int launch_analysis(dfb_state *st, const float *d_audio, int64_t C, int64_t T, float *d_spec, float *d_erb_db,
                     cudaStream_t s, const float *d_init_mem = nullptr, const AnaWindow *w = nullptr);

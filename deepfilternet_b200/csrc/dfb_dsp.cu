@@ -11,9 +11,11 @@
 //   MF.DF                 DeepFilterNet/df/multiframe.py:72-74,126-136,169-180
 //   frame_synthesis       libDF/src/lib.rs:396-427     (pyDF/src/lib.rs:74-107)
 //
-// HBM layout: audio f32[B,T]; spec c64[B,Tf,481] (frame-major, 3848 B rows); features
-// f32[B,Tf,32] and c64[B,Tf,96]; every kernel reads/writes whole rows with consecutive lanes on
-// consecutive addresses.
+// HBM layout: audio f32[B,T]; spec c64[B,Tf,F] (frame-major, F = fft/2 + 1: 481 bins / 3848 B rows at
+// 960 / 480); features f32[B,Tf,E] and c64[B,Tf,nb_df]; every kernel reads/writes whole rows with
+// consecutive lanes on consecutive addresses.
+// Geometry: fft 960 / hop 480 (every shipped model) runs the specialised kernels k_analysis / k_apply_synthesis*;
+// every other supported geometry runs k_analysis_any / k_apply_synthesis_any (runtime mixed-radix FFT).
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -181,7 +183,7 @@ k_analysis(const float *__restrict__ audio, int64_t T, int Tf, float2 *__restric
             pre[q] = v;
         }
         for (int i = tid; i < kFft; i += blockDim.x) s_win[i] = tb.window[i];
-        for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw960[i];
+        for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw_split[i];
         for (int i = tid; i < kN2 * kN1; i += blockDim.x) s_twa[i] = tb.tw_a_fwd[i];
 #pragma unroll
         for (int q = 0; q < kPre; q++) {
@@ -527,15 +529,17 @@ __device__ __forceinline__ float pf_gain_spec(float2 y, float2 x, float beta) {
     return (1.f + beta) / (1.f + beta * q * q);
 }
 
+// F: spectrum row stride (bins); gains_only: this frame takes the ERB gains on every bin (LSNR stage 2)
 __device__ __forceinline__ float2 apply_bin(const ApplyParams &p, const DspTables &tb, const float2 *srow0,
-                                            const float *mrow0, const float *crow, int t, int k) {
+                                            const float *mrow0, const float *crow, int t, int k, int F,
+                                            bool gains_only = false) {
     // srow0 / mrow0: row pointers of frame 0 of this stream
-    float2 x = srow0[(int64_t)t * kF + k];
+    float2 x = srow0[(int64_t)t * F + k];
     float2 y;
     if (p.mode == 0) return x;
     const int band = tb.band_of_bin[k];
     const bool pf2 = p.pf && p.mode == 2;
-    if (k >= p.nb_df || p.mask_only) {
+    if (k >= p.nb_df || p.mask_only || gains_only) {
         float g = mrow0[(int64_t)t * tb.E + band];
         if (pf2) g = pf_gain_mask(g, 0.02f);
         y = make_float2(x.x * g, x.y * g);
@@ -546,7 +550,7 @@ __device__ __forceinline__ float2 apply_bin(const ApplyParams &p, const DspTable
         for (int o = 0; o < p.order; o++) {
             int tt = t + o - (p.order - 1 - p.lookahead);
             if (tt < 0 || tt >= (p.Tv ? p.Tv : p.Tf)) continue;
-            float2 s = srow0[(int64_t)tt * kF + k];
+            float2 s = srow0[(int64_t)tt * F + k];
             if (p.mode == 2 && tt < (p.mc_T ? p.mc_T : p.Tf)) {
                 float g = mrow0[(int64_t)tt * tb.E + band];
                 if (pf2) g = pf_gain_mask(g, 0.02f);
@@ -580,7 +584,7 @@ __global__ void __launch_bounds__(32 * kSynWarps) k_apply_synthesis_generic(Appl
     const int b = blockIdx.y;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int i = tid; i < kFft; i += blockDim.x) s_win[i] = tb.window[i];
-    for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw960[i];
+    for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw_split[i];
     float2 tw[kN1];
 #pragma unroll
     for (int k1 = 0; k1 < kN1; k1++) tw[k1] = lane < kN2 ? tb.tw_a_inv[lane * kN1 + k1] : make_float2(0.f, 0.f);
@@ -607,8 +611,8 @@ __global__ void __launch_bounds__(32 * kSynWarps) k_apply_synthesis_generic(Appl
         for (int j = 0; j < 8; j++) {
             int k = lane + 32 * j;
             if (k <= 240) {
-                float2 xk = apply_bin(p, tb, srow0, mrow0, crow, t, k);
-                float2 xnk = apply_bin(p, tb, srow0, mrow0, crow, t, kC - k);
+                float2 xk = apply_bin(p, tb, srow0, mrow0, crow, t, k, kF);
+                float2 xnk = apply_bin(p, tb, srow0, mrow0, crow, t, kC - k, kF);
                 if (p.spec_out && t >= t0) {
                     float2 *orow = p.spec_out + ((int64_t)b * p.Tf + t) * kF;
                     orow[k] = xk;
@@ -667,7 +671,7 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
     const int b = blockIdx.y;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     for (int i = tid; i < kFft; i += blockDim.x) s_win[i] = tb.window[i];
-    for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw960[i];
+    for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw_split[i];
     for (int i = tid; i < kN2 * kN1; i += blockDim.x) s_twa[i] = tb.tw_a_inv[i];
     __syncthreads();
     const int syn_chunk = p.frames_per_warp ? p.frames_per_warp : kSynChunk;
@@ -820,6 +824,189 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
     }
 }
 
+// ==================================================== every other STFT geometry (fft != 960) ====
+// fft = N = 2 M (M <= 2048 with no prime factor above 7), any hop H <= N / 2.  One warp per frame runs the runtime
+// mixed-radix transform of dfb_fft.cuh in shared memory (dynamic): per CTA the window [N], tw_m [M] and tw_split
+// [M/2 + 1]; per warp two M-point ping-pong buffers and, in the synthesis kernel, the overlap-add memory [N - H].
+constexpr int kAnyAnaWarps = 4, kAnySynWarps = 4;
+// profiler names (dfb_profile_report); constants rather than literals at the launch sites because bench.py's roofline table
+// lists the kernels of the 960 / 480 workloads it runs, and these kernels never run there
+constexpr const char *kAnaAnyName = "k_analysis_any", *kSynAnyName = "k_apply_synthesis_any";
+constexpr int kAnySmemCap = 200 * 1024;   // the synthesis launcher halves its warps per CTA until the CTA fits
+
+__host__ __device__ inline size_t any_align16(size_t b) { return (b + 15) & ~size_t(15); }
+__host__ __device__ inline size_t any_cta_bytes(int N) {
+    const int M = N / 2;
+    return any_align16(sizeof(float) * N) + any_align16(sizeof(float2) * (M + M / 2 + 1));
+}
+__host__ __device__ inline size_t any_warp_bytes(int N, int H, bool syn) {
+    return any_align16(sizeof(float2) * N) + (syn ? any_align16(sizeof(float) * (N - H)) : 0);
+}
+__host__ inline size_t any_smem_bytes(int N, int H, int warps, bool syn) {
+    return any_cta_bytes(N) + (size_t)warps * any_warp_bytes(N, H, syn);
+}
+
+// inverse / forward M-point transform of buffer a (scratch b) by the warp; returns the buffer holding the result
+template <bool INV>
+__device__ __forceinline__ float2 *warp_fft_any(float2 *a, float2 *b, const float2 *tw, int M, int lane) {
+    for (int r = M, Ns = 1; r > 1;) {
+        const int P = fft_next_radix(r);
+        fft_any_pass<INV>(P, a, b, tw, M, Ns, lane, 32);
+        __syncwarp();
+        Ns *= P;
+        r /= P;
+        float2 *t = a; a = b; b = t;
+    }
+    return a;
+}
+
+// per-CTA tables into shared memory; returns the first per-warp byte
+__device__ __forceinline__ unsigned char *any_load_tables(unsigned char *smem, const DspTables &tb, float *&s_win, float2 *&s_twm,
+                                                          float2 *&s_tws) {
+    const int N = tb.fft, M = N / 2;
+    s_win = reinterpret_cast<float *>(smem);
+    s_twm = reinterpret_cast<float2 *>(smem + any_align16(sizeof(float) * N));
+    s_tws = s_twm + M;
+    for (int i = threadIdx.x; i < N; i += blockDim.x) s_win[i] = tb.window[i];
+    for (int i = threadIdx.x; i < M; i += blockDim.x) s_twm[i] = tb.tw_m[i];
+    for (int i = threadIdx.x; i <= M / 2; i += blockDim.x) s_tws[i] = tb.tw_split[i];
+    return smem + any_cta_bytes(N);
+}
+
+// Analysis of any geometry: same arguments and frame window as k_analysis (t_begin, nf, out_t0, Tbuf, row_stride,
+// init_mem).  Frame t covers samples [t H - (N - H), t H + H) (libDF analysis_mem of N - H samples, lib.rs:360-384);
+// init_mem [B][N - H] holds the samples before the stream start (null: zeros).
+// grid (ceil(nf / kAnyAnaWarps), B), block 32 * kAnyAnaWarps.
+// Algorithmic HBM bytes per frame: 4 H R (audio hop) + 8 F W (spec) + 4 E W (erb dB).
+__global__ void __launch_bounds__(32 * kAnyAnaWarps)
+k_analysis_any(const float *__restrict__ audio, int64_t T, int Tf, float2 *__restrict__ spec, float *__restrict__ erb_db,
+               DspTables tb, const float *__restrict__ init_mem, int t_begin, int nf, int out_t0, int Tbuf) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float *s_win;
+    float2 *s_twm, *s_tws;
+    unsigned char *wbase = any_load_tables(smem_raw, tb, s_win, s_twm, s_tws);
+    __syncthreads();
+    const int N = tb.fft, M = N / 2, H = tb.hop, F = tb.F, mem_n = N - H;
+    const int b = blockIdx.y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int tl = blockIdx.x * kAnyAnaWarps + warp, t = t_begin + tl;
+    if (tl >= nf || t >= Tf) return;
+    float2 *A = reinterpret_cast<float2 *>(wbase + (size_t)warp * any_warp_bytes(N, H, false)), *Bf = A + M;
+    const float *x = audio + (int64_t)b * T;
+    const int64_t s0 = (int64_t)t * H - mem_n, s_end = (int64_t)Tf * H;
+    auto sample = [&](int n) -> float {
+        const int64_t i = s0 + n;
+        if (i >= 0) return i < s_end ? __ldg(x + i) : 0.f;
+        return init_mem ? init_mem[(int64_t)b * mem_n + (mem_n + i)] : 0.f;   // carried analysis_mem (reset = False)
+    };
+    for (int n = lane; n < M; n += 32)
+        A[n] = make_float2(sample(2 * n) * s_win[2 * n], sample(2 * n + 1) * s_win[2 * n + 1]);
+    __syncwarp();
+    const float2 *Z = warp_fft_any<false>(A, Bf, s_twm, M, lane);
+    float2 *P2 = Z == A ? Bf : A;   // the free buffer: |X|^2 for the band energies (F <= 2 M floats)
+    float *P = reinterpret_cast<float *>(P2);
+    const int64_t orow = (int64_t)b * Tbuf + out_t0 + tl;
+    float2 *row = spec + orow * F;
+    for (int k = lane; k <= M / 2; k += 32) {
+        float2 xk, xnk;
+        rfft_split(Z[k], Z[(M - k) % M], s_tws[k], xk, xnk);
+        xk.x *= tb.wnorm; xk.y *= tb.wnorm;
+        xnk.x *= tb.wnorm; xnk.y *= tb.wnorm;
+        row[k] = xk;
+        P[k] = __fadd_rn(__fmul_rn(xk.x, xk.x), __fmul_rn(xk.y, xk.y));
+        if (2 * k != M) {
+            row[M - k] = xnk;
+            P[M - k] = __fadd_rn(__fmul_rn(xnk.x, xnk.x), __fmul_rn(xnk.y, xnk.y));
+        }
+    }
+    if (erb_db == nullptr) return;
+    __syncwarp();
+    // band energies: sequential sum inside each band, factor 1/width inside the sum (lib.rs:288-292)
+    for (int band = lane; band < tb.E; band += 32) {
+        int o = tb.erb_off[band], n = tb.erb_off[band + 1] - o;
+        float kinv = tb.erb_kinv[band];
+        float acc = 0.f;
+        for (int j = 0; j < n; j++) acc = __fadd_rn(acc, __fmul_rn(P[o + j], kinv));
+        erb_db[orow * tb.E + band] = __fmul_rn(log10f(__fadd_rn(acc, 1e-10f)), 10.f);
+    }
+}
+
+// Fused apply + synthesis of any geometry: every ApplyParams field of k_apply_synthesis_generic plus the LSNR stage
+// gating of k_apply_synthesis (mode 1).  Overlap-add as libDF frame_synthesis (lib.rs:407-426, S = N - 2 H >= 0):
+//   out[t H + i] = y_t[i] + mem[i] (i < H);  mem <- (mem[H + j] (j < S) or 0) + y_t[H + j]  (j < N - H)
+// One warp owns frames_per_warp consecutive frames and keeps mem in shared memory; it re-synthesises the
+// R = ceil((N - H) / H) frames before its first one to rebuild mem.  With carry (mode 0) the channels form one signal:
+// the re-synthesised frames may lie in the channels before (rows -1, -2, ... of the contiguous [C,Tf,F] spectrum) and
+// the first frame of channel 0 starts from init_tail.
+// Algorithmic HBM bytes per frame (mode 1/2): 8 F R spec + 4 E R m + 8 O nb_df R coefs + 4 H W audio.
+__global__ void __launch_bounds__(32 * kAnySynWarps) k_apply_synthesis_any(ApplyParams p, DspTables tb) {
+    extern __shared__ __align__(16) unsigned char smem_raw[];
+    float *s_win;
+    float2 *s_twm, *s_tws;
+    unsigned char *wbase = any_load_tables(smem_raw, tb, s_win, s_twm, s_tws);
+    __syncthreads();
+    const int N = tb.fft, M = N / 2, H = tb.hop, F = tb.F, mem_n = N - H, S = N - 2 * H, R = (N - 1) / H;
+    const int warps = blockDim.x >> 5;
+    const int b = blockIdx.y, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int t0 = (blockIdx.x * warps + warp) * p.frames_per_warp;
+    if (t0 >= p.Tf) return;
+    const int t1 = min(t0 + p.frames_per_warp, p.Tf);
+    float2 *A = reinterpret_cast<float2 *>(wbase + (size_t)warp * any_warp_bytes(N, H, true)), *Bf = A + M;
+    float *mem = reinterpret_cast<float *>(Bf + M);
+    const float2 *srow0 = p.spec + (int64_t)b * (p.spec_T ? p.spec_T : p.Tf) * F;
+    const int mcT = p.mc_T ? p.mc_T : p.Tf;
+    const float *mrow0 = p.m ? p.m + (int64_t)b * mcT * tb.E : nullptr;
+    const int tmin = p.carry ? -b * p.Tf : 0;   // first frame of the (carried) signal relative to this channel
+    const int tstart = max(t0 - R, tmin);
+    const bool from_init = p.carry && p.init_tail && tstart == tmin;
+    for (int j = lane; j < mem_n; j += 32) mem[j] = from_init ? p.init_tail[j] : 0.f;
+    float *orow = p.audio ? p.audio + (int64_t)b * p.out_stride : nullptr;
+    for (int t = tstart; t < t1; t++) {
+        const float *crow = p.coefs ? p.coefs + ((int64_t)b * mcT + t) * p.nb_df * (2 * p.order) : nullptr;
+        int stage = 3;   // 0 zero gains, 1 unprocessed, 2 gains only, 3 gains + deep filter (tract.rs apply_stages)
+        if (p.lsnr && p.mode == 1) {
+            const float l = p.lsnr[(int64_t)b * mcT + t];
+            stage = l < p.th_min ? 0 : (l > p.th_erb ? 1 : (l > p.th_df ? 2 : 3));
+        }
+        auto bin = [&](int k) -> float2 {
+            if (stage >= 2) return apply_bin(p, tb, srow0, mrow0, crow, t, k, F, stage == 2);
+            const float2 x = srow0[(int64_t)t * F + k];
+            if (stage == 1) return x;
+            return make_float2(x.x * p.atten_lim, x.y * p.atten_lim);   // zero gains, then the attenuation limit
+        };
+        for (int k = lane; k <= M / 2; k += 32) {
+            float2 xk = bin(k), xnk = bin(M - k);
+            if (p.spec_out && t >= t0) {
+                float2 *so = p.spec_out + ((int64_t)b * p.Tf + t) * F;
+                so[k] = xk;
+                so[M - k] = xnk;
+            }
+            if (k == 0) { xk.y = 0.f; xnk.y = 0.f; }  // imag of DC / Nyquist ignored (lib.rs:402)
+            const float2 w = s_tws[k];
+            float2 zk, znk;
+            irfft_merge(xk, xnk, make_float2(w.x, -w.y), zk, znk);
+            A[k] = zk;
+            if (k > 0 && 2 * k != M) A[M - k] = znk;
+        }
+        __syncwarp();
+        if (orow) {
+            float *y = reinterpret_cast<float *>(warp_fft_any<true>(A, Bf, s_twm, M, lane));   // y[n], n < N
+            const bool emit = t >= t0 && t >= p.t_first;
+            for (int i = lane; i < H; i += 32) {
+                const float o = y[i] * s_win[i] + mem[i];     // lib.rs:407-411
+                const int64_t g = (int64_t)t * H + i - p.out_offset;
+                if (emit && g >= 0 && g < p.out_len) orow[g] = o;
+            }
+            for (int j = lane; j < mem_n; j += 32)            // lib.rs:416-426 (rotate_left by H, add, override)
+                y[H + j] = y[H + j] * s_win[H + j] + (j < S ? mem[H + j] : 0.f);
+            __syncwarp();
+            for (int j = lane; j < mem_n; j += 32) mem[j] = y[H + j];
+        }
+        __syncwarp();
+    }
+    if (p.final_tail && b == (int)gridDim.y - 1 && t1 == p.Tf)
+        for (int j = lane; j < mem_n; j += 32) p.final_tail[j] = mem[j];
+}
+
 }  // namespace dfb
 
 // ====================================================================== host side / C ABI ==
@@ -906,9 +1093,14 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
     if (!out) return fail(DFB_ERR_INVALID, "null out");
     *out = nullptr;
     if (hop_size * 2 > fft_size) return fail(DFB_ERR_INVALID, "assertion failed: hop_size * 2 <= fft_size");
-    if (fft_size != kFft || hop_size != kHop)
-        return fail(DFB_ERR_UNSUPPORTED, "built kernels cover fft_size=960, hop_size=480 (got %d, %d)", fft_size,
-                    hop_size);
+    if (hop_size <= 0) return fail(DFB_ERR_INVALID, "hop_size must be positive (got %d)", hop_size);
+    // 960 / 480 runs the specialised kernels; every other geometry the runtime mixed-radix ones
+    const bool spec960 = fft_size == kFft && hop_size == kHop;
+    if (!spec960 && (fft_size % 2 || fft_size < 32 || fft_size > 2 * kAnyMaxM || !fft_any_supported(fft_size / 2)))
+        return fail(DFB_ERR_UNSUPPORTED,
+                    "fft_size %d is not supported: fft_size must be even, 32 <= fft_size <= 4096, and fft_size / 2 must have "
+                    "no prime factor above 7",
+                    fft_size);
     if (nb_erb <= 0 || nb_erb > kMaxErb) return fail(DFB_ERR_INVALID, "nb_erb out of range");
     int rc = use_device(device);
     if (rc) return rc;
@@ -919,7 +1111,7 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
     st->synthesis_mem.assign(fft_size - hop_size, 0.f);
     st->erb.resize(nb_erb);
     dfb_erb_widths(sr, fft_size, nb_erb, min_nb_erb_freqs, st->erb.data());
-    const int F = fft_size / 2 + 1;
+    const int F = fft_size / 2 + 1, M = fft_size / 2;
     // vorbis window, f64 -> f32 (lib.rs:126-132)
     st->window.resize(fft_size);
     const double pi = 3.14159265358979323846;
@@ -927,17 +1119,22 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
         double s = sin(0.5 * pi * ((double)i + 0.5) / (double)(fft_size / 2));
         st->window[i] = (float)sin(0.5 * pi * s * s);
     }
-    // one slab: window | tw_a_fwd | tw_a_inv | tw960 | erb_off | erb_kinv | band_of_bin
-    std::vector<float2> twf(kN2 * kN1), twi(kN2 * kN1), tw960(241);
-    for (int l = 0; l < kN2; l++)
+    // one slab: window | tw_a_fwd | tw_a_inv (960 only) | tw_split | tw_m | erb_off | erb_kinv | band_of_bin
+    const int n_twa = spec960 ? kN2 * kN1 : 0;
+    std::vector<float2> twf(n_twa), twi(n_twa), tw_split(M / 2 + 1), tw_m(M);
+    for (int l = 0; l < kN2 && spec960; l++)
         for (int k1 = 0; k1 < kN1; k1++) {
             double a = 2.0 * pi * (double)((l * k1) % kC) / (double)kC;
             twf[l * kN1 + k1] = make_float2((float)cos(a), (float)-sin(a));
             twi[l * kN1 + k1] = make_float2((float)cos(a), (float)sin(a));
         }
-    for (int k = 0; k <= 240; k++) {
-        double a = 2.0 * pi * (double)k / (double)kFft;
-        tw960[k] = make_float2((float)cos(a), (float)-sin(a));
+    for (int k = 0; k <= M / 2; k++) {
+        double a = 2.0 * pi * (double)k / (double)fft_size;
+        tw_split[k] = make_float2((float)cos(a), (float)-sin(a));
+    }
+    for (int k = 0; k < M; k++) {
+        double a = 2.0 * pi * (double)k / (double)M;
+        tw_m[k] = make_float2((float)cos(a), (float)-sin(a));
     }
     std::vector<int> off(nb_erb + 1, 0);
     std::vector<float> kinv(nb_erb);
@@ -951,15 +1148,17 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
         delete st;
         return fail(DFB_ERR_INVALID, "erb widths sum to %d, expected %d", off[nb_erb], F);
     }
-    size_t o_win = 0, o_twf = o_win + sizeof(float) * fft_size, o_twi = o_twf + sizeof(float2) * twf.size(),
-           o_960 = o_twi + sizeof(float2) * twi.size(), o_off = o_960 + sizeof(float2) * 256,
-           o_kinv = o_off + sizeof(int) * (kMaxErb + 1 + 3), o_bob = o_kinv + sizeof(float) * kMaxErb,
-           total = o_bob + ((F + 255) & ~255);
+    auto a256 = [](size_t b) { return (b + 255) & ~size_t(255); };
+    size_t o_win = 0, o_twf = o_win + a256(sizeof(float) * fft_size), o_twi = o_twf + a256(sizeof(float2) * twf.size()),
+           o_split = o_twi + a256(sizeof(float2) * twi.size()), o_twm = o_split + a256(sizeof(float2) * tw_split.size()),
+           o_off = o_twm + a256(sizeof(float2) * tw_m.size()), o_kinv = o_off + sizeof(int) * (kMaxErb + 1 + 3),
+           o_bob = o_kinv + sizeof(float) * kMaxErb, total = o_bob + a256(F);
     std::vector<char> slab(total, 0);
     memcpy(slab.data() + o_win, st->window.data(), sizeof(float) * fft_size);
     memcpy(slab.data() + o_twf, twf.data(), sizeof(float2) * twf.size());
     memcpy(slab.data() + o_twi, twi.data(), sizeof(float2) * twi.size());
-    memcpy(slab.data() + o_960, tw960.data(), sizeof(float2) * tw960.size());
+    memcpy(slab.data() + o_split, tw_split.data(), sizeof(float2) * tw_split.size());
+    memcpy(slab.data() + o_twm, tw_m.data(), sizeof(float2) * tw_m.size());
     memcpy(slab.data() + o_off, off.data(), sizeof(int) * off.size());
     memcpy(slab.data() + o_kinv, kinv.data(), sizeof(float) * kinv.size());
     memcpy(slab.data() + o_bob, bob.data(), bob.size());
@@ -970,14 +1169,17 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
     }
     st->d_tables = d;
     st->tb.window = (const float *)(d + o_win);
-    st->tb.tw_a_fwd = (const float2 *)(d + o_twf);
-    st->tb.tw_a_inv = (const float2 *)(d + o_twi);
-    st->tb.tw960 = (const float2 *)(d + o_960);
+    st->tb.tw_a_fwd = spec960 ? (const float2 *)(d + o_twf) : nullptr;
+    st->tb.tw_a_inv = spec960 ? (const float2 *)(d + o_twi) : nullptr;
+    st->tb.tw_split = (const float2 *)(d + o_split);
+    st->tb.tw_m = (const float2 *)(d + o_twm);
     st->tb.erb_off = (const int *)(d + o_off);
     st->tb.erb_kinv = (const float *)(d + o_kinv);
     st->tb.band_of_bin = (const unsigned char *)(d + o_bob);
     st->tb.wnorm = 1.f / ((float)((int64_t)fft_size * fft_size) / (float)(2 * hop_size));  // lib.rs:133
     st->tb.fft = fft_size; st->tb.hop = hop_size; st->tb.F = F; st->tb.E = nb_erb;
+    cudaFuncSetAttribute(k_analysis_any, cudaFuncAttributeMaxDynamicSharedMemorySize, kAnySmemCap);
+    cudaFuncSetAttribute(k_apply_synthesis_any, cudaFuncAttributeMaxDynamicSharedMemorySize, kAnySmemCap);
     cudaFuncSetAttribute(k_analysis, cudaFuncAttributeMaxDynamicSharedMemorySize, kAnaSmem);
     if (cudaStreamCreateWithFlags(&st->stream, cudaStreamNonBlocking) != cudaSuccess) {
         cudaFree(d);
@@ -1025,10 +1227,18 @@ int launch_analysis(dfb_state *st, const float *d_audio, int64_t C, int64_t T, f
     if (C > 65535) return fail(DFB_ERR_INVALID, "more than 65535 channels per call");
     const int t_begin = w ? w->t_begin : 0, nf = w ? w->nf : (int)Tf, out_t0 = w ? w->out_t0 : 0, Tbuf = w ? w->Tbuf : (int)Tf;
     if (nf <= 0) return DFB_OK;
-    dim3 grid((unsigned)((nf + kAnaWarps - 1) / kAnaWarps), (unsigned)C);
-    DFB_PROF("k_analysis", s);
-    k_analysis<<<grid, 32 * kAnaWarps, kAnaSmem, s>>>(d_audio, w && w->row_stride ? w->row_stride : T, (int)Tf, (float2 *)d_spec,
-                                                     d_erb_db, st->tb, d_init_mem, t_begin, nf, out_t0, Tbuf);
+    const int64_t row_stride = w && w->row_stride ? w->row_stride : T;
+    if (st->fft == kFft && st->hop == kHop) {
+        dim3 grid((unsigned)((nf + kAnaWarps - 1) / kAnaWarps), (unsigned)C);
+        DFB_PROF("k_analysis", s);
+        k_analysis<<<grid, 32 * kAnaWarps, kAnaSmem, s>>>(d_audio, row_stride, (int)Tf, (float2 *)d_spec, d_erb_db, st->tb,
+                                                         d_init_mem, t_begin, nf, out_t0, Tbuf);
+    } else {
+        dim3 grid((unsigned)((nf + kAnyAnaWarps - 1) / kAnyAnaWarps), (unsigned)C);
+        DFB_PROF(kAnaAnyName, s);
+        k_analysis_any<<<grid, 32 * kAnyAnaWarps, any_smem_bytes(st->fft, st->hop, kAnyAnaWarps, false), s>>>(
+            d_audio, row_stride, (int)Tf, (float2 *)d_spec, d_erb_db, st->tb, d_init_mem, t_begin, nf, out_t0, Tbuf);
+    }
     DFB_LAUNCH_CHECK();
     return DFB_OK;
 }
@@ -1061,11 +1271,25 @@ int launch_feat_norm(const float *d_erb, int E, int64_t erb_stride, const float 
 int launch_apply_synthesis(dfb_state *st, const ApplyParams &p, int64_t B, cudaStream_t s) {
     if (B <= 0 || p.Tf <= 0) return DFB_OK;
     if (B > 65535) return fail(DFB_ERR_INVALID, "more than 65535 channels per call");
-    if (p.mode != 0 && (p.nb_df > 240 || p.order > 8)) return fail(DFB_ERR_UNSUPPORTED, "nb_df > 240 or df_order > 8");
     // frames per warp: 16 amortises the re-synthesis of the frame before a warp's first one; short windows (time chunks)
     // take 8 so that the grid still fills the device with a few waves
     ApplyParams q = p;
     q.frames_per_warp = (B * (int64_t)p.Tf / kSynChunk >= 6000) ? kSynChunk : kSynChunk / 2;
+    if (st->fft != kFft || st->hop != kHop) {
+        if (p.mode != 0 && (p.nb_df > st->tb.F || p.order > 8))
+            return fail(DFB_ERR_UNSUPPORTED, "nb_df > %d bins or df_order > 8", st->tb.F);
+        if (p.lsnr && !(p.mode == 1 && p.m && p.coefs))
+            return fail(DFB_ERR_UNSUPPORTED, "LSNR stage gating is built for DeepFilterNet3 (apply mode 1) only");
+        int warps = kAnySynWarps;
+        while (warps > 1 && any_smem_bytes(st->fft, st->hop, warps, true) > (size_t)kAnySmemCap) warps /= 2;
+        const int per_cta = warps * q.frames_per_warp;
+        dim3 grid((unsigned)((p.Tf + per_cta - 1) / per_cta), (unsigned)B);
+        DFB_PROF(kSynAnyName, s);
+        k_apply_synthesis_any<<<grid, 32 * warps, any_smem_bytes(st->fft, st->hop, warps, true), s>>>(q, st->tb);
+        DFB_LAUNCH_CHECK();
+        return DFB_OK;
+    }
+    if (p.mode != 0 && (p.nb_df > 240 || p.order > 8)) return fail(DFB_ERR_UNSUPPORTED, "nb_df > 240 or df_order > 8");
     int per_cta = kSynWarps * q.frames_per_warp;
     dim3 grid((unsigned)((p.Tf + per_cta - 1) / per_cta), (unsigned)B);
     if (p.lsnr && !(p.mode == 1 && p.order == 5 && p.nb_df == 96 && st->tb.E == 32 && p.m && p.coefs))
@@ -1095,32 +1319,41 @@ extern "C" int dfb_state_reset(dfb_state *st);
 // pyDF DF.analysis(input, reset): reset != 0 starts every channel from zero memory (pyDF/src/lib.rs:56-58);
 // reset == 0 carries the STFT memory from the previous call into channel 0 and from channel c into c + 1
 // (one DFState is shared by all channels).  Either way the memory left behind is the last hop of the last channel.
+// analysis_mem after the frames of one channel: the last fft - hop samples of [mem, x[0, L)) (lib.rs:375-384)
+static void next_analysis_mem(const float *mem, const float *x, int64_t L, int64_t mn, float *out) {
+    for (int64_t j = 0; j < mn; j++) out[j] = L + j < mn ? mem[L + j] : x[L + j - mn];
+}
+
 extern "C" int dfb_analysis_host_ex(dfb_state *st, const float *h_audio, int64_t C, int64_t T, int reset, float *h_spec) {
     if (!st || !h_audio || !h_spec) return fail(DFB_ERR_INVALID, "null argument");
     if (C <= 0 || T <= 0) return fail(DFB_ERR_INVALID, "[df] Input array empty or not contiguous.");
     DFB_CUDA(cudaSetDevice(st->device));
-    const int64_t Tf = T / st->hop, hop = st->hop;
+    const int64_t Tf = T / st->hop, hop = st->hop, mn = st->fft - st->hop;
     if (reset) dfb_state_reset(st);  // DFState::reset clears BOTH memories (libDF/src/lib.rs:156-159)
     size_t nb_in = sizeof(float) * C * T, nb_out = sizeof(float) * 2 * C * Tf * st->tb.F;
-    int rc = st->arena.reserve(nb_in + nb_out + sizeof(float) * C * hop + 2048);
+    int rc = st->arena.reserve(nb_in + nb_out + sizeof(float) * C * mn + 2048);
     if (rc) return rc;
     st->arena.reset();
     float *d_in = st->arena.take<float>(C * T), *d_out = st->arena.take<float>(2 * C * Tf * st->tb.F + 2);
     float *d_mem = nullptr;
     DFB_CUDA(cudaMemcpyAsync(d_in, h_audio, nb_in, cudaMemcpyHostToDevice, st->stream));
+    // memory each channel starts from: channel 0 the carried one, channel c the one channel c - 1 leaves
     std::vector<float> mem;
     if (!reset && Tf > 0) {
-        mem.resize((size_t)C * hop);
-        memcpy(mem.data(), st->analysis_mem.data(), sizeof(float) * hop);
-        for (int64_t c = 1; c < C; c++) memcpy(mem.data() + c * hop, h_audio + (c - 1) * T + (Tf - 1) * hop, sizeof(float) * hop);
-        d_mem = st->arena.take<float>(C * hop);
-        DFB_CUDA(cudaMemcpyAsync(d_mem, mem.data(), sizeof(float) * C * hop, cudaMemcpyHostToDevice, st->stream));
+        mem.resize((size_t)C * mn);
+        memcpy(mem.data(), st->analysis_mem.data(), sizeof(float) * mn);
+        for (int64_t c = 1; c < C; c++) next_analysis_mem(mem.data() + (c - 1) * mn, h_audio + (c - 1) * T, Tf * hop, mn, mem.data() + c * mn);
+        d_mem = st->arena.take<float>(C * mn);
+        DFB_CUDA(cudaMemcpyAsync(d_mem, mem.data(), sizeof(float) * C * mn, cudaMemcpyHostToDevice, st->stream));
     }
     rc = launch_analysis(st, d_in, C, T, d_out, nullptr, st->stream, d_mem);
     if (rc) return rc;
     if (nb_out) DFB_CUDA(cudaMemcpyAsync(h_spec, d_out, nb_out, cudaMemcpyDeviceToHost, st->stream));
     DFB_CUDA(cudaStreamSynchronize(st->stream));
-    if (Tf > 0) memcpy(st->analysis_mem.data(), h_audio + (C - 1) * T + (Tf - 1) * hop, sizeof(float) * hop);
+    if (Tf > 0) {
+        const std::vector<float> start = mem.empty() ? st->analysis_mem : std::vector<float>(mem.end() - mn, mem.end());
+        next_analysis_mem(start.data(), h_audio + (C - 1) * T, Tf * hop, mn, st->analysis_mem.data());
+    }
     return DFB_OK;
 }
 extern "C" int dfb_analysis_host(dfb_state *st, const float *h_audio, int64_t C, int64_t T, float *h_spec) {
@@ -1147,16 +1380,16 @@ extern "C" int dfb_synthesis_host_ex(dfb_state *st, const float *h_spec, int64_t
     if (!st || !h_spec || !h_audio) return fail(DFB_ERR_INVALID, "null argument");
     if (C <= 0 || Tf <= 0) return fail(DFB_ERR_INVALID, "[df] Input array empty or not contiguous.");
     DFB_CUDA(cudaSetDevice(st->device));
-    const int64_t hop = st->hop;
+    const int64_t hop = st->hop, mn = st->fft - st->hop;   // synthesis_mem holds fft - hop samples
     if (reset) dfb_state_reset(st);  // clears the analysis memory as well (libDF/src/lib.rs:156-159)
     size_t nb_in = sizeof(float) * 2 * C * Tf * st->tb.F, nb_out = sizeof(float) * C * Tf * hop;
-    int rc = st->arena.reserve(nb_in + nb_out + sizeof(float) * 2 * hop + 2048);
+    int rc = st->arena.reserve(nb_in + nb_out + sizeof(float) * 2 * mn + 2048);
     if (rc) return rc;
     st->arena.reset();
     float *d_in = st->arena.take<float>(2 * C * Tf * st->tb.F), *d_out = st->arena.take<float>(C * Tf * hop);
-    float *d_init = st->arena.take<float>(hop), *d_final = st->arena.take<float>(hop);
+    float *d_init = st->arena.take<float>(mn), *d_final = st->arena.take<float>(mn);
     DFB_CUDA(cudaMemcpyAsync(d_in, h_spec, nb_in, cudaMemcpyHostToDevice, st->stream));
-    DFB_CUDA(cudaMemcpyAsync(d_init, st->synthesis_mem.data(), sizeof(float) * hop, cudaMemcpyHostToDevice, st->stream));
+    DFB_CUDA(cudaMemcpyAsync(d_init, st->synthesis_mem.data(), sizeof(float) * mn, cudaMemcpyHostToDevice, st->stream));
     ApplyParams p{};
     p.spec = (const float2 *)d_in; p.audio = d_out; p.out_stride = Tf * hop; p.out_offset = 0;
     p.out_len = Tf * hop; p.Tf = (int)Tf; p.mode = 0;
@@ -1164,7 +1397,7 @@ extern "C" int dfb_synthesis_host_ex(dfb_state *st, const float *h_spec, int64_t
     rc = launch_apply_synthesis(st, p, C, st->stream);
     if (rc) return rc;
     DFB_CUDA(cudaMemcpyAsync(h_audio, d_out, nb_out, cudaMemcpyDeviceToHost, st->stream));
-    DFB_CUDA(cudaMemcpyAsync(st->synthesis_mem.data(), d_final, sizeof(float) * hop, cudaMemcpyDeviceToHost, st->stream));
+    DFB_CUDA(cudaMemcpyAsync(st->synthesis_mem.data(), d_final, sizeof(float) * mn, cudaMemcpyDeviceToHost, st->stream));
     DFB_CUDA(cudaStreamSynchronize(st->stream));
     return DFB_OK;
 }

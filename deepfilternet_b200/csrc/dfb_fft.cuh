@@ -1,5 +1,6 @@
-// dfb_fft.cuh -- fp32 FFT building blocks for the 960-point real transforms of the
-// DeepFilterNet analysis / synthesis kernels (sm_100a).
+// dfb_fft.cuh -- fp32 FFT building blocks for the real transforms of the DeepFilterNet analysis /
+// synthesis kernels (sm_100a): the specialised 960-point transform of the shipped models and a
+// runtime mixed-radix transform for every other supported fft_size (end of this file).
 //
 // The reference computes these with realfft 3.3.0 / rustfft 6.2.0 (libDF/src/lib.rs:117-118,
 // :385-388, :398-405): an unnormalised real DFT of length N = fft_size and its inverse.
@@ -9,8 +10,9 @@
 // radix-{2,3,4,5} butterflies with literal twiddles) and the transpose between the two passes
 // goes through a per-warp shared-memory tile.
 //
-// Everything below is __host__ __device__ so that tests/host/fft_host_test.cu can emulate the
-// 32 lanes on the CPU and check the index algebra against a double-precision DFT.
+// Everything below is __host__ __device__ so that tests/host/fft_host_test.cu and
+// tests/host/fft_any_host_test.cu can emulate the 32 lanes on the CPU and check the index algebra
+// against a double-precision DFT.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -152,6 +154,30 @@ struct Dft<5, INV> {
     }
 };
 
+template <bool INV>
+struct Dft<7, INV> {
+    static DFB_HD void run(float2 (&v)[7]) {
+        constexpr float c1 = float(cx_cos2pi(1, 7)), c2 = float(cx_cos2pi(2, 7)), c3 = float(cx_cos2pi(3, 7));
+        constexpr float s1 = float(cx_sin2pi(1, 7)), s2 = float(cx_sin2pi(2, 7)), s3 = float(cx_sin2pi(3, 7));
+        float2 a1 = cadd(v[1], v[6]), a2 = cadd(v[2], v[5]), a3 = cadd(v[3], v[4]);
+        float2 d1 = csub(v[1], v[6]), d2 = csub(v[2], v[5]), d3 = csub(v[3], v[4]);
+        // X[k] = v0 + sum_m cos(2 pi k m / 7) a_m -+ i sum_m sin(2 pi k m / 7) d_m,  X[7-k] with the opposite sign
+        float2 p1 = make_float2(v[0].x + c1 * a1.x + c2 * a2.x + c3 * a3.x, v[0].y + c1 * a1.y + c2 * a2.y + c3 * a3.y);
+        float2 p2 = make_float2(v[0].x + c2 * a1.x + c3 * a2.x + c1 * a3.x, v[0].y + c2 * a1.y + c3 * a2.y + c1 * a3.y);
+        float2 p3 = make_float2(v[0].x + c3 * a1.x + c1 * a2.x + c2 * a3.x, v[0].y + c3 * a1.y + c1 * a2.y + c2 * a3.y);
+        float2 q1 = cmul_mi<INV>(make_float2(s1 * d1.x + s2 * d2.x + s3 * d3.x, s1 * d1.y + s2 * d2.y + s3 * d3.y));
+        float2 q2 = cmul_mi<INV>(make_float2(s2 * d1.x - s3 * d2.x - s1 * d3.x, s2 * d1.y - s3 * d2.y - s1 * d3.y));
+        float2 q3 = cmul_mi<INV>(make_float2(s3 * d1.x - s1 * d2.x + s2 * d3.x, s3 * d1.y - s1 * d2.y + s2 * d3.y));
+        v[0] = cadd(v[0], cadd(a1, cadd(a2, a3)));
+        v[1] = cadd(p1, q1);
+        v[6] = csub(p1, q1);
+        v[2] = cadd(p2, q2);
+        v[5] = csub(p2, q2);
+        v[3] = cadd(p3, q3);
+        v[4] = csub(p3, q3);
+    }
+};
+
 template <int N>
 struct Factor {
     static constexpr int P = (N % 4 == 0) ? 4 : (N % 2 == 0) ? 2 : (N % 3 == 0) ? 3 : (N % 5 == 0) ? 5 : N;
@@ -230,27 +256,87 @@ DFB_HD void fft480_store_natural(const float2 (&b)[kN2], float2* buf, int lane) 
     for (int k2 = 0; k2 < kN2; k2++) buf[lane + kN1 * k2] = b[k2];
 }
 
-// Split step of the real forward transform (N = 960): from Z = DFT480(x[2n] + i x[2n+1]),
-//   X[k] = (Z[k] + conj Z[480-k])/2 - i w960^k (Z[k] - conj Z[480-k])/2,  Z[480] := Z[0]
-// returns X[k] and X[480-k] for one k in [0, 240]; w = e^{-2 pi i k / 960}
+// Split step of the real forward transform of length N = 2 M (960 for the shipped models): from
+// Z = DFT_M(x[2n] + i x[2n+1]),
+//   X[k] = (Z[k] + conj Z[M-k])/2 - i w_N^k (Z[k] - conj Z[M-k])/2,  Z[M] := Z[0]
+// returns X[k] and X[M-k] for one k in [0, M/2]; w = e^{-2 pi i k / N}
 DFB_HD void rfft_split(float2 zk, float2 znk, float2 w, float2& xk, float2& xnk) {
     float2 e = make_float2(0.5f * (zk.x + znk.x), 0.5f * (zk.y - znk.y));   // (Z[k] + conj Z[n-k]) / 2
     float2 d = make_float2(0.5f * (zk.x - znk.x), 0.5f * (zk.y + znk.y));   // (Z[k] - conj Z[n-k]) / 2
     float2 o = cmul(make_float2(d.y, -d.x), w);                             // -i d w
     xk = cadd(e, o);
-    // X[480-k] = conj(e) - conj(o) ... derived from the same pair:  e' = conj(e), d' = -conj(d), w' = -conj(w)
+    // X[M-k] = conj(e) - conj(o) ... derived from the same pair:  e' = conj(e), d' = -conj(d), w' = -conj(w)
     xnk = make_float2(e.x - o.x, -(e.y - o.y));
 }
 
-// Merge step of the real inverse transform: from X[k], X[480-k] (k in [0,240]) build
-//   Z[k] = (X[k] + conj X[480-k]) + i w960^{-k} (X[k] - conj X[480-k])   (unnormalised irfft)
-// and Z[480-k]; wc = e^{+2 pi i k / 960}
+// Merge step of the real inverse transform: from X[k], X[M-k] (k in [0, M/2]) build
+//   Z[k] = (X[k] + conj X[M-k]) + i w_N^{-k} (X[k] - conj X[M-k])   (unnormalised irfft)
+// and Z[M-k]; wc = e^{+2 pi i k / N}
 DFB_HD void irfft_merge(float2 xk, float2 xnk, float2 wc, float2& zk, float2& znk) {
     float2 e = make_float2(xk.x + xnk.x, xk.y - xnk.y);
     float2 d = make_float2(xk.x - xnk.x, xk.y + xnk.y);
     float2 o = cmul(make_float2(-d.y, d.x), wc);  // i d wc
     zk = cadd(e, o);
     znk = make_float2(e.x - o.x, -(e.y - o.y));
+}
+
+// ------------------------------------------------ runtime mixed-radix transform (any M) ----
+// The analysis / synthesis kernels of every other STFT geometry (k_analysis_any, k_apply_synthesis_any) run the
+// M = fft_size / 2 point complex transform as a Stockham autosort FFT in shared memory: one pass per radix of the plan
+// (fft_next_radix), natural order in and out, ping-pong between two M-point buffers.  One code path serves
+// every supported size; the radix of a pass is a runtime switch over the compile-time butterflies above.
+constexpr int kAnyMaxM = 2048;     // fft_size <= 4096
+
+// radix of the next pass for the remaining length r (4 first, then 2, 3, 5, 7); 0: a prime factor above 7 is left
+DFB_HD int fft_next_radix(int r) {
+    return r % 4 == 0 ? 4 : r % 2 == 0 ? 2 : r % 3 == 0 ? 3 : r % 5 == 0 ? 5 : r % 7 == 0 ? 7 : 0;
+}
+inline bool fft_any_supported(int M) {
+    if (M < 1 || M > kAnyMaxM) return false;
+    while (M > 1) {
+        const int p = fft_next_radix(M);
+        if (!p) return false;
+        M /= p;
+    }
+    return true;
+}
+
+// One radix-P pass (Stockham, decimation in time).  Ns = product of the radices of the earlier passes; butterfly
+// j < M/P of lane `lane` (stride nlanes):
+//   v_r = src[j + r M/P] * w_{Ns P}^{-+ r (j mod Ns)},  v = DFT_P(v),  dst[(j - j mod Ns) P + j mod Ns + r Ns] = v_r
+// tw[k] = e^{-2 pi i k / M} (w_{Ns P}^{m} = tw[m M / (Ns P)]); the inverse conjugates it.
+template <int P, bool INV>
+DFB_HD void stockham_pass(const float2 *src, float2 *dst, const float2 *tw, int M, int Ns, int lane, int nlanes) {
+    const int q = M / P, tstep = M / (Ns * P);
+    for (int j = lane; j < q; j += nlanes) {
+        const int jm = j % Ns;
+        float2 v[P];
+#pragma unroll
+        for (int r = 0; r < P; r++) {
+            float2 x = src[j + r * q];
+            if (r > 0 && jm > 0) {
+                float2 w = tw[jm * r * tstep];
+                if (INV) w.y = -w.y;
+                x = cmul(x, w);
+            }
+            v[r] = x;
+        }
+        Dft<P, INV>::run(v);
+        const int d = (j - jm) * P + jm;
+#pragma unroll
+        for (int r = 0; r < P; r++) dst[d + r * Ns] = v[r];
+    }
+}
+
+template <bool INV>
+DFB_HD void fft_any_pass(int P, const float2 *src, float2 *dst, const float2 *tw, int M, int Ns, int lane, int nlanes) {
+    switch (P) {
+        case 4: stockham_pass<4, INV>(src, dst, tw, M, Ns, lane, nlanes); break;
+        case 2: stockham_pass<2, INV>(src, dst, tw, M, Ns, lane, nlanes); break;
+        case 3: stockham_pass<3, INV>(src, dst, tw, M, Ns, lane, nlanes); break;
+        case 5: stockham_pass<5, INV>(src, dst, tw, M, Ns, lane, nlanes); break;
+        default: stockham_pass<7, INV>(src, dst, tw, M, Ns, lane, nlanes); break;
+    }
 }
 
 }  // namespace dfb

@@ -1826,6 +1826,8 @@ extern "C" int dfb_model_set_chunking(dfb_model *m, int device_chunks, int host_
 // The workspace is sized from the model's band layout but the DSP kernels index with the state's: they must agree.
 static int check_state(const dfb_model *m, const dfb_state *st) {
     if (m->device != st->device) return fail(DFB_ERR_INVALID, "model and state live on different devices");
+    if (m->cfg.nb_df > st->tb.F)
+        return fail(DFB_ERR_INVALID, "nb_df = %d exceeds the %d frequency bins of fft_size %d", m->cfg.nb_df, st->tb.F, st->fft);
     if (st->tb.E != m->cfg.nb_erb)
         return fail(DFB_ERR_INVALID, "DF state has %d ERB bands, the model was built for %d", st->tb.E, m->cfg.nb_erb);
     if (!m->erb_widths.empty())
@@ -1833,6 +1835,15 @@ static int check_state(const dfb_model *m, const dfb_state *st) {
             if (m->erb_widths[i] != st->erb[i])
                 return fail(DFB_ERR_INVALID, "DF state's ERB band %d is %lld bins wide, the model was built for %lld", i,
                             (long long)st->erb[i], (long long)m->erb_widths[i]);
+    return DFB_OK;
+}
+
+// The time-chunked executor carries one hop of STFT memory and one frame of overlap-add tail per stream, which is the
+// whole state only when hop == fft / 2 (every DeepFilterNet config).
+static int check_half_overlap(const dfb_state *st) {
+    if (st->hop * 2 != st->fft)
+        return fail(DFB_ERR_UNSUPPORTED, "enhance / streaming need hop_size == fft_size / 2 (got fft_size %d, hop_size %d); "
+                    "use analysis, DfNet.forward and synthesis for other hops", st->fft, st->hop);
     return DFB_OK;
 }
 
@@ -2225,6 +2236,7 @@ extern "C" int dfb_enhance(dfb_model *m, dfb_state *st, const float *d_audio, in
     if (!m || !st || !d_audio || !d_out) return fail(DFB_ERR_INVALID, "null argument");
     if (B <= 0 || T <= 0) return fail(DFB_ERR_INVALID, "empty input");
     if (int rcs = check_state(m, st)) return rcs;
+    if (int rch = check_half_overlap(st)) return rch;
     DFB_CUDA(cudaSetDevice(m->device));
     cudaStream_t s = (cudaStream_t)stream;
     const int hop = st->hop, fft = st->fft;
@@ -2272,6 +2284,7 @@ extern "C" int dfb_enhance_host(dfb_model *m, dfb_state *st, const float *h_audi
     if (!m || !st || !h_audio || !h_out) return fail(DFB_ERR_INVALID, "null argument");
     if (B <= 0 || T <= 0) return fail(DFB_ERR_INVALID, "empty input");
     if (int rcs = check_state(m, st)) return rcs;
+    if (int rch = check_half_overlap(st)) return rch;
     DFB_CUDA(cudaSetDevice(m->device));
     const int hop = st->hop, fft = st->fft;
     const int64_t Tp = pad ? T + fft : T, Tf = Tp / hop;
@@ -2358,6 +2371,7 @@ extern "C" int dfb_stream_create(dfb_stream **out, dfb_model *m, dfb_state *st, 
     if (!out || !m || !st || B <= 0 || B > 65535) return fail(DFB_ERR_INVALID, "bad argument");
     *out = nullptr;
     if (int rcs = check_state(m, st)) return rcs;
+    if (int rch = check_half_overlap(st)) return rch;
     if (m->cfg.model_kind == 1)
         return fail(DFB_ERR_UNSUPPORTED, "DeepFilterNet v1 runs as one window per signal (forward_v1): no frame-incremental API");
     DFB_CUDA(cudaSetDevice(m->device));

@@ -8,7 +8,10 @@ Differences kept on purpose (documented in INTEGRATION.md):
     ``unsafe as_array_mut``, pyDF/src/lib.rs:87,262);
   * ``reset=False`` carries the STFT / ISTFT memories across calls and channels exactly like the
     reference's shared ``DFState`` (channel 0 continues the previous call, channel c continues c - 1);
-  * only fft_size=960 / hop_size=480 kernels are built (all shipped models).
+  * STFT geometries: 960 / 480 (every shipped model) runs specialised kernels; any other even
+    fft_size with 32 <= fft_size <= 4096 and no prime factor above 7 in fft_size / 2 (320, 384,
+    512, 640, 882, 1024, 1920, 4096, ...) runs the runtime mixed-radix kernels, for every
+    hop_size <= fft_size / 2.  Other sizes raise ``DfbError`` (DFB_ERR_UNSUPPORTED).
 """
 from __future__ import annotations
 

@@ -81,6 +81,9 @@ class DfNet(nn.Module):
         if (self.df_state.nb_erb() != cfg.nb_erb or self.df_state.fft_size() != cfg.fft_size
                 or self.df_state.hop_size() != cfg.hop_size):
             raise ValueError("df_state was built with a different nb_erb / fft_size / hop_size than the model config")
+        if cfg.nb_df > cfg.fft_size // 2 + 1:
+            raise _lib.DfbError(_lib.DFB_ERR_INVALID, f"nb_df = {cfg.nb_df} exceeds the {cfg.fft_size // 2 + 1} frequency "
+                                                      f"bins of fft_size {cfg.fft_size}")
         self.df_state.norm_alpha = cfg.norm_alpha  # read by df_features (enhance.py:192)
         # keep the reference tensors (state_dict() parity); buffers, not parameters: inference only
         self._sd_names = []

@@ -58,7 +58,12 @@ int64_t dfb_profile_report(char *buf, int64_t buflen);
 typedef struct dfb_state dfb_state;
 
 /* pyDF DF.__new__ (pyDF/src/lib.rs:22-39) -> DFState::new (libDF/src/lib.rs:104-154).
- * device: CUDA ordinal.  Built kernels: fft_size 960 / hop_size 480 (all shipped models). */
+ * device: CUDA ordinal.  STFT geometries: fft_size 960 / hop_size 480 (all shipped models) runs specialised
+ * kernels; any other even fft_size with 32 <= fft_size <= 4096 whose half has no prime factor above 7 (320, 384,
+ * 512, 640, 882, 1024, 1920, 4096, ...) runs runtime mixed-radix kernels, at any hop_size <= fft_size / 2 for
+ * analysis / synthesis / features / forward / apply.  Other sizes: DFB_ERR_UNSUPPORTED; hop_size * 2 > fft_size:
+ * DFB_ERR_INVALID.  dfb_enhance* and dfb_stream_* need hop_size == fft_size / 2 (DFB_ERR_UNSUPPORTED otherwise);
+ * a model whose nb_df exceeds fft_size / 2 + 1 is rejected with DFB_ERR_INVALID. */
 int dfb_state_create(dfb_state **out, int device, int sr, int fft_size, int hop_size, int nb_erb,
                      int min_nb_erb_freqs);
 void dfb_state_free(dfb_state *st);
