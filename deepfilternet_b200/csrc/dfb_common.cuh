@@ -106,11 +106,11 @@ struct Arena {
 
 constexpr int kMaxErb = 64;
 
-// Device-resident tables of one DSP state.  M = fft / 2; the 960 / 480 kernels read tw_a_*, every other geometry the
-// runtime FFT (dfb_fft.cuh) with tw_m.
+// Device-resident tables of one DSP state.  M = fft / 2; the specialised 960 / 480 kernels (k_analysis,
+// k_apply_synthesis) read tw_a_*, the runtime FFT (dfb_fft.cuh) of every other kernel tw_m.
 struct DspTables {
     const float *window;     // [fft]
-    const float2 *tw_a_fwd;  // [24][20]  w480^{-lane k1} (fft 960 only, else null)
+    const float2 *tw_a_fwd;  // [24][20]  w480^{-lane k1} (960 / 480 only, else null)
     const float2 *tw_a_inv;  // [24][20]  conj
     const float2 *tw_split;  // [M/2 + 1] e^{-2 pi i k / fft}  (real split / merge steps)
     const float2 *tw_m;      // [M]       e^{-2 pi i k / M}    (runtime FFT passes)

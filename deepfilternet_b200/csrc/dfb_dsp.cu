@@ -14,8 +14,9 @@
 // HBM layout: audio f32[B,T]; spec c64[B,Tf,F] (frame-major, F = fft/2 + 1: 481 bins / 3848 B rows at
 // 960 / 480); features f32[B,Tf,E] and c64[B,Tf,nb_df]; every kernel reads/writes whole rows with
 // consecutive lanes on consecutive addresses.
-// Geometry: fft 960 / hop 480 (every shipped model) runs the specialised kernels k_analysis / k_apply_synthesis*;
-// every other supported geometry runs k_analysis_any / k_apply_synthesis_any (runtime mixed-radix FFT).
+// Geometry: fft 960 / hop 480 (every shipped model) runs the specialised kernels k_analysis and, for the shipped models'
+// apply shape, k_apply_synthesis; every other supported geometry, and 960 / 480's plain ISTFT and other apply shapes, run
+// k_analysis_any / k_apply_synthesis_any (runtime mixed-radix FFT).
 #include <cmath>
 #include <cstdlib>
 #include <cstring>
@@ -106,15 +107,16 @@ constexpr int kAnaSmem = sizeof(float) * ((kAnaWarps + 1) * 480 + 960) + sizeof(
 // One warp: 480-point complex FFT of the values gathered by `load(n)` (n = 24 n1 + lane), result
 // in natural order in buf[0..480).  `buf` is a per-warp shared buffer of kTileFloat2 float2 that
 // serves as the pass-A/B transpose tile and then as the natural-order output; `load` may read it.
+// tw_lane -> the 20 pass-A twiddles of this lane (shared memory).
 template <bool INV, typename LoadF>
-__device__ __forceinline__ void warp_fft480(LoadF load, const float2 (&tw)[kN1], float2 *buf, int lane) {
+__device__ __forceinline__ void warp_fft480(LoadF load, const float2 *tw_lane, float2 *buf, int lane) {
     float2 a[kN1];
     if (lane < kN2) {
 #pragma unroll
         for (int n1 = 0; n1 < kN1; n1++) a[n1] = load(kN2 * n1 + lane);
     }
     __syncwarp();
-    if (lane < kN2) fft480_pass_a<INV>(a, tw, buf, lane);
+    if (lane < kN2) fft480_pass_a<INV>(a, tw_lane, buf, lane);
     __syncwarp();
     float2 b[kN2];
     if (lane < kN1) fft480_pass_b<INV>(b, buf, lane);
@@ -123,22 +125,16 @@ __device__ __forceinline__ void warp_fft480(LoadF load, const float2 (&tw)[kN1],
     __syncwarp();
 }
 
-// variant with the pass-A twiddles of this lane read from memory (tw_lane -> 20 float2)
-template <bool INV, typename LoadF>
-__device__ __forceinline__ void warp_fft480_twptr(LoadF load, const float2 *tw_lane, float2 *buf, int lane) {
-    float2 a[kN1];
-    if (lane < kN2) {
-#pragma unroll
-        for (int n1 = 0; n1 < kN1; n1++) a[n1] = load(kN2 * n1 + lane);
+// ERB band energies of one frame from its power spectrum P, in dB, to out[0..E): sequential sum inside each band, factor
+// 1/width inside the sum (lib.rs:288-292)
+__device__ __forceinline__ void erb_band_db(const float *P, const DspTables &tb, float *out, int lane) {
+    for (int band = lane; band < tb.E; band += 32) {
+        int o = tb.erb_off[band], n = tb.erb_off[band + 1] - o;
+        float kinv = tb.erb_kinv[band];
+        float acc = 0.f;
+        for (int j = 0; j < n; j++) acc = __fadd_rn(acc, __fmul_rn(P[o + j], kinv));
+        out[band] = __fmul_rn(log10f(__fadd_rn(acc, 1e-10f)), 10.f);
     }
-    __syncwarp();
-    if (lane < kN2) fft480_pass_a_ptr<INV>(a, tw_lane, buf, lane);
-    __syncwarp();
-    float2 b[kN2];
-    if (lane < kN1) fft480_pass_b<INV>(b, buf, lane);
-    __syncwarp();
-    if (lane < kN1) fft480_store_natural(b, buf, lane);
-    __syncwarp();
 }
 
 // ---------------------------------------------------------------------------- analysis ----
@@ -197,7 +193,7 @@ k_analysis(const float *__restrict__ audio, int64_t T, int Tf, float2 *__restric
     const int64_t orow = (int64_t)b * Tbuf + out_t0 + tl0 + warp;   // row of this frame in the output buffers
     const float *fr = s_stage + warp * kHop;  // frame t = samples [(t-1) hop, (t+1) hop)
     float2 *nat = s_buf + warp * kTileFloat2;
-    warp_fft480_twptr<false>(
+    warp_fft480<false>(
         [&](int n) {
             float2 v = *reinterpret_cast<const float2 *>(fr + 2 * n);
             float2 w = *reinterpret_cast<const float2 *>(s_win + 2 * n);
@@ -235,14 +231,7 @@ k_analysis(const float *__restrict__ audio, int64_t T, int Tf, float2 *__restric
         }
     }
     __syncwarp();
-    // band energies: sequential sum inside each band, factor 1/width inside the sum (lib.rs:288-292)
-    for (int band = lane; band < tb.E; band += 32) {
-        int o = tb.erb_off[band], n = tb.erb_off[band + 1] - o;
-        float kinv = tb.erb_kinv[band];
-        float acc = 0.f;
-        for (int j = 0; j < n; j++) acc = __fadd_rn(acc, __fmul_rn(P[o + j], kinv));
-        erb_db[orow * tb.E + band] = __fmul_rn(log10f(__fadd_rn(acc, 1e-10f)), 10.f);
-    }
+    erb_band_db(P, tb, erb_db + orow * tb.E, lane);
 }
 
 // ----------------------------------------------------------- generic ERB (libdf.erb) ----
@@ -577,93 +566,26 @@ __device__ __forceinline__ float2 apply_bin(const ApplyParams &p, const DspTable
     return y;
 }
 
-__global__ void __launch_bounds__(32 * kSynWarps) k_apply_synthesis_generic(ApplyParams p, DspTables tb) {
-    __shared__ __align__(16) float s_win[kFft];
-    __shared__ __align__(16) float2 s_tw960[241];
-    __shared__ __align__(16) float2 s_buf[kSynWarps][kTileFloat2];
-    const int b = blockIdx.y;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int i = tid; i < kFft; i += blockDim.x) s_win[i] = tb.window[i];
-    for (int i = tid; i < 241; i += blockDim.x) s_tw960[i] = tb.tw_split[i];
-    float2 tw[kN1];
-#pragma unroll
-    for (int k1 = 0; k1 < kN1; k1++) tw[k1] = lane < kN2 ? tb.tw_a_inv[lane * kN1 + k1] : make_float2(0.f, 0.f);
-    __syncthreads();
-    const int syn_chunk = p.frames_per_warp ? p.frames_per_warp : kSynChunk;
-    const int t0 = (blockIdx.x * kSynWarps + warp) * syn_chunk;
-    if (t0 >= p.Tf) return;
-    const int t1 = min(t0 + syn_chunk, p.Tf);
-    const float2 *srow0 = p.spec + (int64_t)b * (p.spec_T ? p.spec_T : p.Tf) * kF;
-    const int mcT = p.mc_T ? p.mc_T : p.Tf;
-    const float *mrow0 = p.m ? p.m + (int64_t)b * mcT * tb.E : nullptr;
-    float2 *nat = s_buf[warp];
-    float *yb = reinterpret_cast<float *>(nat);  // 960 windowed samples of the current frame
-    float tail[15];
-#pragma unroll
-    for (int j = 0; j < 15; j++) tail[j] = (p.carry && t0 == 0 && b == 0 && p.init_tail) ? p.init_tail[lane + 32 * j] : 0.f;
-    // carried state: channel b > 0 continues from the tail of channel b - 1's last frame, which is row -1
-    // relative to this channel in the contiguous [C,Tf,F] spectrum (mode 0 only)
-    const int tstart = t0 > 0 ? t0 - 1 : ((p.carry && b > 0) ? -1 : 0);
-    for (int t = tstart; t < t1; t++) {
-        const float *crow = p.coefs ? p.coefs + ((int64_t)b * mcT + t) * p.nb_df * (2 * p.order) : nullptr;
-        // gather X[k], X[480-k], merge into Z (natural order in `nat`)
-#pragma unroll
-        for (int j = 0; j < 8; j++) {
-            int k = lane + 32 * j;
-            if (k <= 240) {
-                float2 xk = apply_bin(p, tb, srow0, mrow0, crow, t, k, kF);
-                float2 xnk = apply_bin(p, tb, srow0, mrow0, crow, t, kC - k, kF);
-                if (p.spec_out && t >= t0) {
-                    float2 *orow = p.spec_out + ((int64_t)b * p.Tf + t) * kF;
-                    orow[k] = xk;
-                    orow[kC - k] = xnk;
-                }
-                if (k == 0) { xk.y = 0.f; xnk.y = 0.f; }  // imag of DC / Nyquist ignored (lib.rs:402)
-                float2 w = s_tw960[k];
-                float2 zk, znk;
-                irfft_merge(xk, xnk, make_float2(w.x, -w.y), zk, znk);
-                nat[k] = zk;
-                if (k > 0 && k < 240) nat[kC - k] = znk;
-            }
-        }
-        __syncwarp();
-        if (p.audio) {
-            // reads of nat complete inside pass A before pass B overwrites it (warp syncs inside)
-            warp_fft480<true>([&](int n) { return nat[n]; }, tw, nat, lane);
-            // nat[n] = (x[2n], x[2n+1]); window in place
-#pragma unroll
-            for (int j = 0; j < 15; j++) {
-                int n = lane + 32 * j;
-                float2 v = nat[n];
-                float2 w = *reinterpret_cast<const float2 *>(s_win + 2 * n);
-                nat[n] = make_float2(v.x * w.x, v.y * w.y);
-            }
-            __syncwarp();
-            float *orow = p.audio + (int64_t)b * p.out_stride;
-#pragma unroll
-            for (int j = 0; j < 15; j++) {
-                int i = lane + 32 * j;
-                float o = yb[i] + tail[j];      // lib.rs:407-411
-                tail[j] = yb[kHop + i];         // lib.rs:423-426 (hop == fft/2)
-                int64_t g = (int64_t)t * kHop + i - p.out_offset;
-                if (t >= t0 && t >= p.t_first && g >= 0 && g < p.out_len) orow[g] = o;
-            }
-        }
-        __syncwarp();
+// LSNR stage of frame row i (tract.rs apply_stages): 0 zero gains, 1 unprocessed, 2 gains only, 3 gains + deep filter
+__device__ __forceinline__ int lsnr_stage(const ApplyParams &p, int64_t i) {
+    int stage = 3;
+    if (p.lsnr) {
+        const float l = p.lsnr[i];
+        stage = l < p.th_min ? 0 : (l > p.th_erb ? 1 : (l > p.th_df ? 2 : 3));
     }
-    if (p.final_tail && b == (int)gridDim.y - 1 && t1 == p.Tf) {
-#pragma unroll
-        for (int j = 0; j < 15; j++) p.final_tail[lane + 32 * j] = tail[j];
-    }
+    return stage;
 }
 
-// Specialised version for the shipped models (df_order 5, nb_df 96, 32 ERB bands): a lane owns the bins
+// apply shape of the shipped models: df_order 5, nb_df 96 = 3 DF bins per lane, 32 ERB bands
+constexpr int kOrder = 5, kNdfj = 3, kBands = 32;
+
+// Specialised version for the shipped models' apply shape at 960 / 480: a lane owns the bins
 // k = lane + 32 j (and 480 - k) for every frame of its chunk, so the deep-filter input history of its DF
 // bins lives in registers as a 5-deep shift register (one new look-ahead value per bin and frame instead of
 // five reloads), the band gains come from one register per lane via warp shuffles, and all global loads of
 // a frame are issued up front, coalesced (256-byte rows), before any use.
-template <int ORDER, int NDFJ, int MINB>
-__global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyParams p, DspTables tb) {
+// 2 CTAs / SM (no spills) measured fastest.
+__global__ void __launch_bounds__(32 * kSynWarps, 2) k_apply_synthesis(ApplyParams p, DspTables tb) {
     __shared__ __align__(16) float s_win[kFft];
     __shared__ __align__(16) float2 s_tw960[241];
     __shared__ __align__(16) float2 s_buf[kSynWarps][kTileFloat2];
@@ -678,11 +600,11 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
     const int t0 = (blockIdx.x * kSynWarps + warp) * syn_chunk;
     if (t0 >= p.Tf) return;
     const int t1 = min(t0 + syn_chunk, p.Tf);
-    const int Tf = p.Tf, L = p.lookahead, back = ORDER - 1 - L;
+    const int Tf = p.Tf, L = p.lookahead, back = kOrder - 1 - L;
     const int Tv = p.Tv ? p.Tv : Tf;                       // spectrum rows >= Tv do not exist (end of the stream)
     const float2 *srow0 = p.spec + (int64_t)b * (p.spec_T ? p.spec_T : Tf) * kF;
     const int mcT = p.mc_T ? p.mc_T : Tf;                  // m / coefs rows per stream
-    const float *mrow0 = p.m + (int64_t)b * mcT * 32;
+    const float *mrow0 = p.m + (int64_t)b * mcT * kBands;
     const bool masked_df = p.mode == 2 && !p.mask_only;
     const bool pf1 = p.pf && p.mode == 1, pf2 = p.pf && p.mode == 2;
     const bool blend = p.alpha != nullptr && masked_df;   // DeepFilterNet v1: alpha blend with the masked bin
@@ -703,51 +625,47 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
 #pragma unroll
     for (int j = 0; j < 15; j++) tail[j] = 0.f;
     // S'[tt][k] for the DF bins; tt = t + o - back.  Rows outside [0, Tf) are zero (multiframe.py:72-74).
-    auto load_df_row = [&](int tt, float2 (&dst)[NDFJ]) {
+    auto load_df_row = [&](int tt, float2 (&dst)[kNdfj]) {
         float g = 1.f;
         const bool ok = tt >= 0 && tt < Tv;
         // (DFN2) the mask of a look-ahead frame beyond the window's DNN frames does not exist yet: such rows are only
         // read for frames that are re-synthesised in the next window
-        float mrow = (ok && masked_df && tt < mcT) ? mrow0[(int64_t)tt * 32 + lane] : 1.f;
+        float mrow = (ok && masked_df && tt < mcT) ? mrow0[(int64_t)tt * kBands + lane] : 1.f;
         if (pf2 && ok && masked_df && tt < mcT) mrow = pf_gain_mask(mrow, 0.02f);
 #pragma unroll
-        for (int j = 0; j < NDFJ; j++) {
+        for (int j = 0; j < kNdfj; j++) {
             float2 v = ok ? srow0[(int64_t)tt * kF + lane + 32 * j] : make_float2(0.f, 0.f);
             if (masked_df) { g = __shfl_sync(0xffffffffu, mrow, BK(j)); v.x *= g; v.y *= g; }
             dst[j] = v;
         }
     };
     const int tstart = t0 > 0 ? t0 - 1 : 0;
-    float2 hist[ORDER][NDFJ];
+    float2 hist[kOrder][kNdfj];
 #pragma unroll
-    for (int o = 1; o < ORDER; o++) load_df_row(tstart + o - 1 - back, hist[o]);  // becomes taps 0..O-2 after the first shift
+    for (int o = 1; o < kOrder; o++) load_df_row(tstart + o - 1 - back, hist[o]);  // becomes taps 0..O-2 after the first shift
     for (int t = tstart; t < t1; t++) {
         // ---- loads of this frame, all issued before use
-        float mcur = mrow0[(int64_t)t * 32 + lane];
+        float mcur = mrow0[(int64_t)t * kBands + lane];
         if (pf2) mcur = pf_gain_mask(mcur, 0.02f);
         const float al = blend ? p.alpha[(int64_t)b * mcT + t] : 1.f;
-        int stage = 3;   // 0 zero gains, 1 unprocessed, 2 gains only, 3 gains + deep filter (tract.rs apply_stages)
-        if (p.lsnr) {
-            const float l = p.lsnr[(int64_t)b * mcT + t];
-            stage = l < p.th_min ? 0 : (l > p.th_erb ? 1 : (l > p.th_df ? 2 : 3));
-        }
+        const int stage = lsnr_stage(p, (int64_t)b * mcT + t);
 #pragma unroll
-        for (int o = 0; o < ORDER - 1; o++)
+        for (int o = 0; o < kOrder - 1; o++)
 #pragma unroll
-            for (int j = 0; j < NDFJ; j++) hist[o][j] = hist[o + 1][j];
-        load_df_row(t + L, hist[ORDER - 1]);
-        float2 cf[NDFJ][ORDER];
-        const float2 *crow = reinterpret_cast<const float2 *>(p.coefs + ((int64_t)b * mcT + t) * (NDFJ * 32) * (2 * ORDER));
+            for (int j = 0; j < kNdfj; j++) hist[o][j] = hist[o + 1][j];
+        load_df_row(t + L, hist[kOrder - 1]);
+        float2 cf[kNdfj][kOrder];
+        const float2 *crow = reinterpret_cast<const float2 *>(p.coefs + ((int64_t)b * mcT + t) * (kNdfj * 32) * (2 * kOrder));
 #pragma unroll
-        for (int j = 0; j < NDFJ; j++)
+        for (int j = 0; j < kNdfj; j++)
 #pragma unroll
-            for (int o = 0; o < ORDER; o++) cf[j][o] = crow[(lane + 32 * j) * ORDER + o];
+            for (int o = 0; o < kOrder; o++) cf[j][o] = crow[(lane + 32 * j) * kOrder + o];
         float2 xk[8], xn[8];
         const float2 *srow = srow0 + (int64_t)t * kF;
 #pragma unroll
         for (int j = 0; j < 8; j++) {
             const int k = lane + 32 * j;
-            xk[j] = (k <= 240 && (j >= NDFJ || need_xk)) ? srow[k] : make_float2(0.f, 0.f);
+            xk[j] = (k <= 240 && (j >= kNdfj || need_xk)) ? srow[k] : make_float2(0.f, 0.f);
             xn[j] = k <= 240 ? srow[kC - k] : make_float2(0.f, 0.f);
         }
         // ---- deep filter (bins < 96), gain (others), optional attenuation limit
@@ -755,10 +673,10 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
         for (int j = 0; j < 8; j++) {
             const int k = lane + 32 * j;
             float2 y;
-            if (j < NDFJ && !p.mask_only && stage == 3) {
+            if (j < kNdfj && !p.mask_only && stage == 3) {
                 float yr = 0.f, yi = 0.f;
 #pragma unroll
-                for (int o = 0; o < ORDER; o++) {
+                for (int o = 0; o < kOrder; o++) {
                     const float2 s = hist[o][j], w = cf[j][o];
                     yr += s.x * w.x - s.y * w.y;
                     yi += s.x * w.y + s.y * w.x;
@@ -801,7 +719,7 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
         }
         __syncwarp();
         if (p.audio) {
-            warp_fft480_twptr<true>([&](int n) { return nat[n]; }, s_twa + (lane < kN2 ? lane : 0) * kN1, nat, lane);
+            warp_fft480<true>([&](int n) { return nat[n]; }, s_twa + (lane < kN2 ? lane : 0) * kN1, nat, lane);
 #pragma unroll
             for (int j = 0; j < 15; j++) {
                 int n = lane + 32 * j;
@@ -824,7 +742,7 @@ __global__ void __launch_bounds__(32 * kSynWarps, MINB) k_apply_synthesis(ApplyP
     }
 }
 
-// ==================================================== every other STFT geometry (fft != 960) ====
+// ================================================== runtime mixed-radix kernels (any geometry) ====
 // fft = N = 2 M (M <= 2048 with no prime factor above 7), any hop H <= N / 2.  One warp per frame runs the runtime
 // mixed-radix transform of dfb_fft.cuh in shared memory (dynamic): per CTA the window [N], tw_m [M] and tw_split
 // [M/2 + 1]; per warp two M-point ping-pong buffers and, in the synthesis kernel, the overlap-add memory [N - H].
@@ -920,18 +838,12 @@ k_analysis_any(const float *__restrict__ audio, int64_t T, int Tf, float2 *__res
     }
     if (erb_db == nullptr) return;
     __syncwarp();
-    // band energies: sequential sum inside each band, factor 1/width inside the sum (lib.rs:288-292)
-    for (int band = lane; band < tb.E; band += 32) {
-        int o = tb.erb_off[band], n = tb.erb_off[band + 1] - o;
-        float kinv = tb.erb_kinv[band];
-        float acc = 0.f;
-        for (int j = 0; j < n; j++) acc = __fadd_rn(acc, __fmul_rn(P[o + j], kinv));
-        erb_db[orow * tb.E + band] = __fmul_rn(log10f(__fadd_rn(acc, 1e-10f)), 10.f);
-    }
+    erb_band_db(P, tb, erb_db + orow * tb.E, lane);
 }
 
-// Fused apply + synthesis of any geometry: every ApplyParams field of k_apply_synthesis_generic plus the LSNR stage
-// gating of k_apply_synthesis (mode 1).  Overlap-add as libDF frame_synthesis (lib.rs:407-426, S = N - 2 H >= 0):
+// Fused apply + synthesis of any geometry, for every apply shape and every ApplyParams field, including the LSNR stage
+// gating (mode 1); at 960 / 480 it serves the plain ISTFT and the shapes k_apply_synthesis is not specialised for.
+// Overlap-add as libDF frame_synthesis (lib.rs:407-426, S = N - 2 H >= 0):
 //   out[t H + i] = y_t[i] + mem[i] (i < H);  mem <- (mem[H + j] (j < S) or 0) + y_t[H + j]  (j < N - H)
 // One warp owns frames_per_warp consecutive frames and keeps mem in shared memory; it re-synthesises the
 // R = ceil((N - H) / H) frames before its first one to rebuild mem.  With carry (mode 0) the channels form one signal:
@@ -962,11 +874,7 @@ __global__ void __launch_bounds__(32 * kAnySynWarps) k_apply_synthesis_any(Apply
     float *orow = p.audio ? p.audio + (int64_t)b * p.out_stride : nullptr;
     for (int t = tstart; t < t1; t++) {
         const float *crow = p.coefs ? p.coefs + ((int64_t)b * mcT + t) * p.nb_df * (2 * p.order) : nullptr;
-        int stage = 3;   // 0 zero gains, 1 unprocessed, 2 gains only, 3 gains + deep filter (tract.rs apply_stages)
-        if (p.lsnr && p.mode == 1) {
-            const float l = p.lsnr[(int64_t)b * mcT + t];
-            stage = l < p.th_min ? 0 : (l > p.th_erb ? 1 : (l > p.th_df ? 2 : 3));
-        }
+        const int stage = lsnr_stage(p, (int64_t)b * mcT + t);
         auto bin = [&](int k) -> float2 {
             if (stage >= 2) return apply_bin(p, tb, srow0, mrow0, crow, t, k, F, stage == 2);
             const float2 x = srow0[(int64_t)t * F + k];
@@ -1094,7 +1002,7 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
     *out = nullptr;
     if (hop_size * 2 > fft_size) return fail(DFB_ERR_INVALID, "assertion failed: hop_size * 2 <= fft_size");
     if (hop_size <= 0) return fail(DFB_ERR_INVALID, "hop_size must be positive (got %d)", hop_size);
-    // 960 / 480 runs the specialised kernels; every other geometry the runtime mixed-radix ones
+    // 960 / 480 has specialised kernels; every other geometry needs a size the runtime mixed-radix FFT supports
     const bool spec960 = fft_size == kFft && hop_size == kHop;
     if (!spec960 && (fft_size % 2 || fft_size < 32 || fft_size > 2 * kAnyMaxM || !fft_any_supported(fft_size / 2)))
         return fail(DFB_ERR_UNSUPPORTED,
@@ -1119,7 +1027,8 @@ extern "C" int dfb_state_create(dfb_state **out, int device, int sr, int fft_siz
         double s = sin(0.5 * pi * ((double)i + 0.5) / (double)(fft_size / 2));
         st->window[i] = (float)sin(0.5 * pi * s * s);
     }
-    // one slab: window | tw_a_fwd | tw_a_inv (960 only) | tw_split | tw_m | erb_off | erb_kinv | band_of_bin
+    // one slab: window | tw_a_fwd | tw_a_inv (960 / 480 only: the specialised kernels) | tw_split | tw_m | erb_off | erb_kinv |
+    // band_of_bin
     const int n_twa = spec960 ? kN2 * kN1 : 0;
     std::vector<float2> twf(n_twa), twi(n_twa), tw_split(M / 2 + 1), tw_m(M);
     for (int l = 0; l < kN2 && spec960; l++)
@@ -1251,8 +1160,7 @@ int launch_feat_norm(const float *d_erb, int E, int64_t erb_stride, const float 
     if (E + Fd > 1024) return fail(DFB_ERR_INVALID, "E + F > 1024 in norm scan");
     int threads = ((E + Fd + 31) / 32) * 32;
     DFB_PROF("k_feat_norm", s);
-    static const bool no_seg = getenv("DFB_NORM_SEG") && !atoi(getenv("DFB_NORM_SEG"));
-    if (threads <= 128 && Tf >= 16 * kNormSeg && !no_seg)
+    if (threads <= 128 && Tf >= 16 * kNormSeg)
         k_feat_norm_seg<<<(unsigned)C, 128 * kNormSeg, 0, s>>>(d_erb, E, erb_stride, (const float2 *)d_spec, Fd, spec_stride, (int)Tf,
                                                             alpha, d_erb_state, d_unit_state, d_feat_erb, (float2 *)d_feat_spec,
                                                             (int)(Ts > 0 ? Ts : Tf), d_erb_state_out, d_unit_state_out);
@@ -1271,37 +1179,28 @@ int launch_feat_norm(const float *d_erb, int E, int64_t erb_stride, const float 
 int launch_apply_synthesis(dfb_state *st, const ApplyParams &p, int64_t B, cudaStream_t s) {
     if (B <= 0 || p.Tf <= 0) return DFB_OK;
     if (B > 65535) return fail(DFB_ERR_INVALID, "more than 65535 channels per call");
+    if (p.mode != 0 && (p.nb_df > st->tb.F || p.order > 8))
+        return fail(DFB_ERR_UNSUPPORTED, "nb_df > %d bins or df_order > 8", st->tb.F);
+    if (p.lsnr && !(p.mode == 1 && p.m && p.coefs))
+        return fail(DFB_ERR_UNSUPPORTED, "LSNR stage gating is built for DeepFilterNet3 (apply mode 1) only");
     // frames per warp: 16 amortises the re-synthesis of the frame before a warp's first one; short windows (time chunks)
     // take 8 so that the grid still fills the device with a few waves
     ApplyParams q = p;
     q.frames_per_warp = (B * (int64_t)p.Tf / kSynChunk >= 6000) ? kSynChunk : kSynChunk / 2;
-    if (st->fft != kFft || st->hop != kHop) {
-        if (p.mode != 0 && (p.nb_df > st->tb.F || p.order > 8))
-            return fail(DFB_ERR_UNSUPPORTED, "nb_df > %d bins or df_order > 8", st->tb.F);
-        if (p.lsnr && !(p.mode == 1 && p.m && p.coefs))
-            return fail(DFB_ERR_UNSUPPORTED, "LSNR stage gating is built for DeepFilterNet3 (apply mode 1) only");
+    if (st->fft == kFft && st->hop == kHop && p.mode != 0 && p.order == kOrder && p.nb_df == 32 * kNdfj && st->tb.E == kBands &&
+        p.m && p.coefs) {
+        const int per_cta = kSynWarps * q.frames_per_warp;
+        dim3 grid((unsigned)((p.Tf + per_cta - 1) / per_cta), (unsigned)B);
+        DFB_PROF("k_apply_synthesis", s);
+        k_apply_synthesis<<<grid, 32 * kSynWarps, 0, s>>>(q, st->tb);
+    } else {
         int warps = kAnySynWarps;
         while (warps > 1 && any_smem_bytes(st->fft, st->hop, warps, true) > (size_t)kAnySmemCap) warps /= 2;
         const int per_cta = warps * q.frames_per_warp;
         dim3 grid((unsigned)((p.Tf + per_cta - 1) / per_cta), (unsigned)B);
         DFB_PROF(kSynAnyName, s);
         k_apply_synthesis_any<<<grid, 32 * warps, any_smem_bytes(st->fft, st->hop, warps, true), s>>>(q, st->tb);
-        DFB_LAUNCH_CHECK();
-        return DFB_OK;
     }
-    if (p.mode != 0 && (p.nb_df > 240 || p.order > 8)) return fail(DFB_ERR_UNSUPPORTED, "nb_df > 240 or df_order > 8");
-    int per_cta = kSynWarps * q.frames_per_warp;
-    dim3 grid((unsigned)((p.Tf + per_cta - 1) / per_cta), (unsigned)B);
-    if (p.lsnr && !(p.mode == 1 && p.order == 5 && p.nb_df == 96 && st->tb.E == 32 && p.m && p.coefs))
-        return fail(DFB_ERR_UNSUPPORTED, "LSNR stage gating is built for the DeepFilterNet3 apply kernel only");
-    DFB_PROF("k_apply_synthesis", s);
-    static const int minb = getenv("DFB_APPLY_MINB") ? atoi(getenv("DFB_APPLY_MINB")) : 2;  // 2 CTAs/SM without spills measured fastest
-    if (p.mode != 0 && p.order == 5 && p.nb_df == 96 && st->tb.E == 32 && p.m && p.coefs && minb == 3)
-        k_apply_synthesis<5, 3, 3><<<grid, 32 * kSynWarps, 0, s>>>(q, st->tb);
-    else if (p.mode != 0 && p.order == 5 && p.nb_df == 96 && st->tb.E == 32 && p.m && p.coefs && minb == 2)
-        k_apply_synthesis<5, 3, 2><<<grid, 32 * kSynWarps, 0, s>>>(q, st->tb);
-    else
-        k_apply_synthesis_generic<<<grid, 32 * kSynWarps, 0, s>>>(q, st->tb);
     DFB_LAUNCH_CHECK();
     return DFB_OK;
 }

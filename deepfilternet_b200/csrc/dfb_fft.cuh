@@ -227,17 +227,9 @@ constexpr int kN1 = 20, kN2 = 24;
 constexpr int kTileStride = 25;  // float2 units; 25 keeps the pass-B column reads conflict free
 constexpr int kTileFloat2 = kN1 * kTileStride;  // 500 float2 = 4000 B per warp
 
-// Pass A for one lane.  `a` holds z[24 n1 + lane] (n1 = 0..19); `tw` = w480^{-+ lane k1}.
+// Pass A for one lane.  `a` holds z[24 n1 + lane] (n1 = 0..19); `tw` -> w480^{-+ lane k1} (k1 = 0..19), e.g. in shared memory.
 template <bool INV>
-DFB_HD void fft480_pass_a(float2 (&a)[kN1], const float2 (&tw)[kN1], float2* tile, int lane) {
-    Dft<kN1, INV>::run(a);
-#pragma unroll
-    for (int k1 = 0; k1 < kN1; k1++) tile[k1 * kTileStride + lane] = cmul(a[k1], tw[k1]);
-}
-
-// Same with the twiddles read through a pointer (e.g. shared memory) instead of held in registers.
-template <bool INV>
-DFB_HD void fft480_pass_a_ptr(float2 (&a)[kN1], const float2* tw, float2* tile, int lane) {
+DFB_HD void fft480_pass_a(float2 (&a)[kN1], const float2* tw, float2* tile, int lane) {
     Dft<kN1, INV>::run(a);
 #pragma unroll
     for (int k1 = 0; k1 < kN1; k1++) tile[k1 * kTileStride + lane] = cmul(a[k1], tw[k1]);

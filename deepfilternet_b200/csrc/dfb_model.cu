@@ -1428,8 +1428,7 @@ static int forward_body(dfb_model *m, Arena &arena, const float *d_feat_erb, con
                         c.df_pathway_kt);
         if (Fd % 2) return fail(DFB_ERR_UNSUPPORTED, "df pathway conv: odd nb_df");
         dim3 grid((unsigned)((Fd + 2 * kCpWarps - 1) / (2 * kCpWarps)), (unsigned)((T + kCpChunk - 1) / kCpChunk), (unsigned)B);
-        static const bool convp_ffma = getenv("DFB_CONVP_FFMA") && atoi(getenv("DFB_CONVP_FFMA"));
-        const float *w_sw = (m->conv_tc && !convp_ffma) ? m->get("df_dec.df_convp.w_sw") : nullptr;
+        const float *w_sw = m->conv_tc ? m->get("df_dec.df_convp.w_sw") : nullptr;
         if (w_sw) {  // channel contraction on tcgen05 (BF16x3), shifted adds + 1x1 conv in the epilogue
             if ((rc = launch_df_convp_tc(sl, f.c0, w_sw, w2, bb, d_coefs, B, T, Fd))) return rc;
         } else {
@@ -1498,11 +1497,9 @@ static int forward_body(dfb_model *m, Arena &arena, const float *d_feat_erb, con
     // DFN3's grouped-linear skip around the DF GRU does not depend on the recurrence: evaluate it here (the ERB
     // branch has the slack) and let the last GRU layer add it as its output residual, instead of a kernel on the
     // DF branch's tail, which is the critical path of the decoder phase
-    // the two decoders' recurrences run concurrently and at most 15 clusters of 8 CTAs are co-resident: one branch uses 32
-    // streams per cluster for batches above 64 (DFB_WIDE_BRANCH=erb|df|both|none selects which, for experiments)
-    static const char *wide_env = getenv("DFB_WIDE_BRANCH");
-    const int wide_df = !wide_env || !strcmp(wide_env, "df") || !strcmp(wide_env, "both");
-    const int wide_erb = wide_env && (!strcmp(wide_env, "erb") || !strcmp(wide_env, "both"));
+    // the two decoders' recurrences run concurrently and at most 15 clusters of 8 CTAs are co-resident: the DF branch uses 32
+    // streams per cluster for batches above 64, the ERB branch 16
+    const int wide_df = 1, wide_erb = 0;
     const bool early_skip = c.g_df_skip && c.model_kind != 2;
     if (early_skip) {
         if ((rc = gl(s, "df_dec.df_skip.gl", f.emb, emb_dim, &pl_emb, c.g_df_skip, emb_dim, Hd, ACT_NONE, nullptr, 0, f.dfskip, Hd, nullptr)))

@@ -296,19 +296,6 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
     for (int i = 0; i < 16; i++) v[i] = __uint_as_float(r[i]);
 }
 
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t saddr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-    return r;
-}
-
-// bulk copy own shared memory -> a peer CTA's shared memory, completing `bytes` on the peer's mbarrier
-__device__ __forceinline__ void dsmem_bulk_copy(uint32_t dst_cluster, uint32_t src_cta, uint32_t bytes, uint32_t mbar_cluster) {
-    asm volatile("cp.async.bulk.shared::cluster.shared::cta.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(dst_cluster),
-                 "r"(src_cta), "r"(bytes), "r"(mbar_cluster)
-                 : "memory");
-}
-
 // global -> the same shared-memory offset of every CTA of the cluster named in cta_mask; completes `bytes` on the mbarrier at
 // the same offset in each of them
 __device__ __forceinline__ void bulk_load_multicast(uint32_t dst, const void *src, uint32_t bytes, uint32_t bar, uint16_t cta_mask) {

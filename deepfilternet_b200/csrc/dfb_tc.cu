@@ -656,11 +656,12 @@ __global__ void __launch_bounds__(kCvThreads, 2) k_df_convp_tc(const __grid_cons
 // CTA's 32 units are one contiguous 2 KB piece).  Per time step one warp issues 48 tcgen05.mma
 // (TS mode: A from TMEM, B from smem; M128 N16 K16, kind::f16: hi*hi + lo*hi + hi*lo, fp32
 // accumulate in TMEM); eight warps read the pre-activations from TMEM, apply the gates in fp32,
-// write the CTA's slice of the new state into its own operand buffer and broadcast it with one
-// bulk DSMEM copy per peer (cp.async.bulk shared::cta -> shared::cluster) that completes bytes on
-// the peer's mbarrier -- no cluster barrier or fence on the step's critical path.  The fp32 hidden
-// state of a CTA's own units stays in registers; only the MMA operand is BF16.
-// Measured step timeline (clock64, 16 streams, XG = 1, profiles/r02_gru_anatomy.txt): 48 MMAs 450 cycles, commit ->
+// store the CTA's slice of the new state to a global scratch piece, and one thread asks the TMA
+// engine for a multicast bulk copy of that piece into the operand buffer of every CTA of the
+// cluster (itself included), which completes bytes on each CTA's mbarrier -- no cluster barrier
+// on the step's critical path.  The fp32 hidden state of a CTA's own units stays in registers;
+// only the MMA operand is BF16.
+// Measured step timeline (clock64, 16 streams, profiles/r02_gru_anatomy.txt): 48 MMAs 450 cycles, commit ->
 // gates 135, TMEM load + gates 645, fence 39, barrier + multicast through L2 + global stores 984  =>  2090 cycles / step
 // (round 1, DSMEM exchange: 2380; the FFMA kernel k_gru: 4700).  History of the issue loop: `if (lane == 0)` around each
 // MMA ~50 cycles per instruction (ptxas wrapped each in an ELECT / R2UR / BRA.U.ANY loop); every lane executing every
@@ -670,7 +671,7 @@ namespace cg = cooperative_groups;
 constexpr int kGtU = 32, kGtRows = 3 * kGtU;   // hidden units / W_hh rows per CTA (both hidden sizes)
 // gate threads: one per (unit pair, stream) item = 16 * NS; plus the MMA warp
 // h operand (B, K-major, no swizzle) as 8 x 16 B core matrices ordered [k core matrix][row group][hi|lo]:
-// a CTA's 32 units (4 k core matrices) are one contiguous piece (2 KB for 16 streams) -> one bulk DSMEM copy per peer.
+// a CTA's 32 units (4 k core matrices) are one contiguous piece (2 KB for 16 streams) -> one multicast bulk copy.
 // NS = streams per cluster (MMA N): 16 (lowest step latency) or 32 (half as many clusters: the DF decoder's
 // recurrence uses it for large batches so that it is co-resident with the ERB decoder's -- at most 15 clusters
 // of 8 CTAs fit on the device, and two launches of 8 clusters made the second one run in two waves).
@@ -726,15 +727,14 @@ struct GruTcParams {
     int t0, Ts;
     int B, T, Bc;
     long long *dbg;      // optional [T][8] clock64 stamps of CTA 0 (0-3: MMA thread, 4-7: gate thread 0)
-    unsigned char *xbuf; // (XG) exchange scratch in global memory [cluster][2][CTA][kPiece]
+    unsigned char *xbuf; // exchange scratch in global memory [cluster][2][CTA][kPiece]
 };
 
 
-// XG = 1: the new state travels through L2 instead of SM to SM -- every CTA stores its slice to a global scratch piece and
-// asks the TMA engine for ONE multicast bulk copy of that piece into all CTAs of the cluster (itself included); the
-// per-peer DSMEM copies (15 x 4 KB out and in per CTA and step at H = 512 / 32 streams, ~20 B/cycle on the SM-to-SM
-// network: more than half of the step) become one 4 KB read that the crossbar replicates.
-template <int NS, int HH, int XG>
+// The new state travels through L2 instead of SM to SM: per-peer DSMEM copies (15 x 4 KB out and in per CTA and step at
+// H = 512 / 32 streams, ~20 B/cycle on the SM-to-SM network: more than half of the step) become one 4 KB read that the
+// crossbar replicates.
+template <int NS, int HH>
 __global__ void __launch_bounds__(GtCfg<NS, HH>::kThreads, 1) k_gru_tc(GruTcParams p) {
     using Cfg = GtCfg<NS, HH>;
     constexpr int kGtThreads = Cfg::kThreads;
@@ -750,8 +750,8 @@ __global__ void __launch_bounds__(GtCfg<NS, HH>::kThreads, 1) k_gru_tc(GruTcPara
     const int H = kGtH, T = p.T;
     for (int i = tid; i < (int)sizeof(sm.h) / 16; i += kGtThreads) reinterpret_cast<uint4 *>(&sm.h[0][0])[i] = make_uint4(0, 0, 0, 0);  // h0 = 0
     if (tid == 0) {
-        mbar_init(&sm.bar_h[0], XG ? 1 : 2);   // MMA thread's expect_tx arrive (+ one gate-warp arrive: own slice written)
-        mbar_init(&sm.bar_h[1], XG ? 1 : 2);
+        mbar_init(&sm.bar_h[0], 1);   // MMA thread's expect_tx arrive
+        mbar_init(&sm.bar_h[1], 1);
         mbar_init(&sm.t_full, 1);
         fence_barrier_init();
     }
@@ -812,7 +812,7 @@ __global__ void __launch_bounds__(GtCfg<NS, HH>::kThreads, 1) k_gru_tc(GruTcPara
     __syncthreads();
     tc_fence_after();
     cluster.sync();  // every CTA's barriers are initialised and its h buffers zeroed before any remote copy
-    const uint32_t step_bytes = (uint32_t)((kGtC - (XG ? 0 : 1)) * Cfg::kPiece);  // one piece from each of the peers (XG: and the own one)
+    const uint32_t step_bytes = (uint32_t)(kGtC * Cfg::kPiece);  // one piece from each CTA of the cluster, itself included
 
     if (warp == Cfg::kMmaWarp) {
         // ================================================================= MMA issuer (whole warp, elected lane issues)
@@ -921,38 +921,22 @@ __global__ void __launch_bounds__(GtCfg<NS, HH>::kThreads, 1) k_gru_tc(GruTcPara
                 bf16_split(hprev1, h1, l1);
                 vhi = h0 | (uint32_t)h1 << 16;
                 vlo = l0 | (uint32_t)l1 << 16;
-                if (t + 1 < T) {
-                    if (XG) {   // own piece of the scratch buffer (same layout as the shared-memory slice)
-                        unsigned char *xp = p.xbuf + ((size_t)(group * 2 + (cur ^ 1)) * kGtC + rank) * Cfg::kPiece + (hoff - piece0);
-                        *reinterpret_cast<uint32_t *>(xp) = vhi;
-                        *reinterpret_cast<uint32_t *>(xp + Cfg::kPlane) = vlo;
-                    } else {
-                        *reinterpret_cast<uint32_t *>(sm.h[cur ^ 1] + hoff) = vhi;
-                        *reinterpret_cast<uint32_t *>(sm.h[cur ^ 1] + hoff + Cfg::kPlane) = vlo;
-                    }
+                if (t + 1 < T) {   // own piece of the scratch buffer (same layout as the shared-memory slice)
+                    unsigned char *xp = p.xbuf + ((size_t)(group * 2 + (cur ^ 1)) * kGtC + rank) * Cfg::kPiece + (hoff - piece0);
+                    *reinterpret_cast<uint32_t *>(xp) = vhi;
+                    *reinterpret_cast<uint32_t *>(xp + Cfg::kPlane) = vlo;
                 }
             }
             if (gdbg) p.dbg[t * 8 + 6] = clock64();
             if (t + 1 < T) {
-                // own slice (generic stores) -> visible to the bulk-copy / tensor-core proxy
-                if (XG) fence_proxy_async_global(); else fence_proxy_async();
+                // own slice (generic stores) -> visible to the bulk-copy proxy
+                fence_proxy_async_global();
                 if (gdbg) p.dbg[t * 8 + 3] = clock64();
                 asm volatile("bar.sync 1, %0;" ::"n"(Cfg::kGateThreads) : "memory");
-                if (XG) {
-                    if (tid == 0) {
-                        const unsigned char *xp = p.xbuf + ((size_t)(group * 2 + (cur ^ 1)) * kGtC + rank) * Cfg::kPiece;
-                        bulk_load_multicast(smem_u32(sm.h[cur ^ 1]) + piece0, xp, Cfg::kPiece, smem_u32(&sm.bar_h[cur ^ 1]),
-                                            (uint16_t)((1u << kGtC) - 1u));
-                    }
-                } else if (lane == 0) {
-                    // gate warp w copies the CTA's slice to peers w, w + #warps, ... (skipping itself); the last gate warp
-                    // also signals the local barrier
-                    const uint32_t src = smem_u32(sm.h[cur ^ 1]) + piece0;
-                    for (int j = warp; j < kGtC - 1; j += Cfg::kGateWarps) {
-                        const int peer = j + (j >= rank ? 1 : 0);
-                        dsmem_bulk_copy(mapa_u32(src, peer), src, Cfg::kPiece, mapa_u32(smem_u32(&sm.bar_h[cur ^ 1]), peer));
-                    }
-                    if (warp == Cfg::kGateWarps - 1) mbar_arrive(&sm.bar_h[cur ^ 1]);  // own slice is in place
+                if (tid == 0) {
+                    const unsigned char *xp = p.xbuf + ((size_t)(group * 2 + (cur ^ 1)) * kGtC + rank) * Cfg::kPiece;
+                    bulk_load_multicast(smem_u32(sm.h[cur ^ 1]) + piece0, xp, Cfg::kPiece, smem_u32(&sm.bar_h[cur ^ 1]),
+                                        (uint16_t)((1u << kGtC) - 1u));
                 }
             } else {
                 asm volatile("bar.sync 1, %0;" ::"n"(Cfg::kGateThreads) : "memory");
@@ -979,7 +963,7 @@ __global__ void __launch_bounds__(GtCfg<NS, HH>::kThreads, 1) k_gru_tc(GruTcPara
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-// exchange scratch of the XG variant: one buffer per (device, stream) -- launches on one stream are serialised, the two
+// exchange scratch of the recurrence: one buffer per (device, stream) -- launches on one stream are serialised, the two
 // decoders' recurrences run on different streams
 static unsigned char *gru_xbuf(cudaStream_t s, size_t bytes) {
     struct Ent { unsigned char *p = nullptr; size_t cap = 0; };
@@ -998,7 +982,7 @@ static unsigned char *gru_xbuf(cudaStream_t s, size_t bytes) {
     return e.p;
 }
 
-template <int NS, int HH, int XG>
+template <int NS, int HH>
 static int launch_gru_tc_n(cudaStream_t s, GruTcParams p) {
     using Cfg = GtCfg<NS, HH>;
     static PerDeviceOnce attr_once;
@@ -1010,8 +994,8 @@ static int launch_gru_tc_n(cudaStream_t s, GruTcParams p) {
     // tcgen05.alloc -- no change at 128 x 10 s with 1 .. 4 device chunks, 512 x 10 s: 45.2 vs 45.3 ms)
     const int smem = need > 120 * 1024 ? need : 120 * 1024;
     if (auto once_guard = attr_once.first()) {
-        if (Cfg::kC > 8) DFB_CUDA(cudaFuncSetAttribute(k_gru_tc<NS, HH, XG>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        DFB_CUDA(cudaFuncSetAttribute(k_gru_tc<NS, HH, XG>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        if (Cfg::kC > 8) DFB_CUDA(cudaFuncSetAttribute(k_gru_tc<NS, HH>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+        DFB_CUDA(cudaFuncSetAttribute(k_gru_tc<NS, HH>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     }
     cudaLaunchConfig_t cfg{};
     cfg.blockDim = dim3(Cfg::kThreads);
@@ -1024,12 +1008,10 @@ static int launch_gru_tc_n(cudaStream_t s, GruTcParams p) {
     const int ngroups = (p.B + NS - 1) / NS;
     cfg.gridDim = dim3((unsigned)(ngroups * Cfg::kC));
     cfg.stream = s;
-    if (XG) {
-        p.xbuf = gru_xbuf(s, (size_t)ngroups * 2 * Cfg::kC * Cfg::kPiece);
-        if (!p.xbuf) return fail(DFB_ERR_OOM, "GRU exchange scratch");
-    }
+    p.xbuf = gru_xbuf(s, (size_t)ngroups * 2 * Cfg::kC * Cfg::kPiece);
+    if (!p.xbuf) return fail(DFB_ERR_OOM, "GRU exchange scratch");
     DFB_PROF(HH == 256 ? "k_gru_tc" : "k_gru_tc512", s);
-    DFB_CUDA(cudaLaunchKernelEx(&cfg, k_gru_tc<NS, HH, XG>, p));
+    DFB_CUDA(cudaLaunchKernelEx(&cfg, k_gru_tc<NS, HH>, p));
     g_launches.fetch_add(1, std::memory_order_relaxed);
     return DFB_OK;
 }
@@ -1041,34 +1023,25 @@ int launch_gru_tc(cudaStream_t s, const float *xproj, const float *whh, const fl
                   const GruWindow *w, int H) {
     GruTcParams p{xproj, whh, bhh, res, hout, hout_hi, hout_lo, planes_res, w ? w->h0 : nullptr, w ? w->hT : nullptr,
                   w ? w->t0 : 0, w ? w->Ts : T, B, T, 0, dbg};
-    static const int force = getenv("DFB_GRU_NS") ? atoi(getenv("DFB_GRU_NS")) : 0;
     // (Tried: a "ping-pong" kernel in which a cluster owns 2 or 3 independent sub-batches of 16 streams -- own state buffers,
     // accumulator columns, barriers and 8 gate warps each, one MMA warp serving them in turn -- so that one sub-batch's
     // MMAs fill the other's gate / exchange latency.  Correct (parity tests green), but 48 MMAs of N = 16 take ~800 cycles to
     // issue (16.7 per instruction, twice their math time), so two sub-batches keep the MMA warp busy 1800 of the 2650-cycle
     // chain and the chain itself stretches: 3127 cycles per step for 2 x 16 streams vs 3050 for one N = 32 batch, 3947 for
     // 3 x 16; 128 x 10 s 11.75 vs 11.31 ms.)
-    // exchange through L2 + multicast (k_gru_tc XG): bit 0: H = 512, bit 1: H = 256 / 32 streams, bit 2: H = 256 / 16 streams.
-    // Measured: H = 512 256 x 10 s 60.8 -> 51.0 ms, 32 x 10 s 12.0 -> 9.5 ms; H = 256 / 32 streams: 512 x 10 s 43.9 -> 41.6 ms;
-    // H = 256 / 16 streams: 128 x 10 s 11.88 -> 11.34 ms, 32 x 10 s 5.57 -> 5.09 ms, batch 1 3.79 -> 3.62 ms.  Default: all.
-    static const int xg = getenv("DFB_GRU_XG") ? atoi(getenv("DFB_GRU_XG")) : 7;
-    if (H == 512) {
-        const bool n32 = force ? force == 32 : B > 128;
-        if (xg & 1) return n32 ? launch_gru_tc_n<32, 512, 1>(s, p) : launch_gru_tc_n<16, 512, 1>(s, p);
-        return n32 ? launch_gru_tc_n<32, 512, 0>(s, p) : launch_gru_tc_n<16, 512, 0>(s, p);
-    }
+    // exchange through L2 + multicast instead of per-peer DSMEM copies, measured: H = 512 256 x 10 s 60.8 -> 51.0 ms,
+    // 32 x 10 s 12.0 -> 9.5 ms; H = 256 / 32 streams: 512 x 10 s 43.9 -> 41.6 ms; H = 256 / 16 streams: 128 x 10 s
+    // 11.88 -> 11.34 ms, 32 x 10 s 5.57 -> 5.09 ms, batch 1 3.79 -> 3.62 ms.
+    if (H == 512) return B > 128 ? launch_gru_tc_n<32, 512>(s, p) : launch_gru_tc_n<16, 512>(s, p);
     if (H != 256) return fail(DFB_ERR_UNSUPPORTED, "tensor-core recurrence: hidden size %d", H);
     // 16 streams per cluster have the shortest step (2600 cycles vs 3830 for 32) but 36 % more cluster time per stream:
     // from 256 streams on a launch needs several waves of the 15 co-resident clusters anyway, and 32 per cluster are faster
     // (512 x 10 s DeepFilterNet2: 48.1 -> 45.3 ms per step)
-    const bool use32 = force ? force == 32 : ((wide && B > 64) || B >= 256);
+    const bool use32 = (wide && B > 64) || B >= 256;
     // beyond 15 x 32 streams a launch of 32-stream clusters needs a second wave of the 15 co-resident clusters (512 streams:
     // 16 clusters -> twice the time); 48 streams per cluster (N = 48, 768 gate threads) keep 512 streams in one wave
-    static const int no48 = getenv("DFB_GRU_NO48") ? atoi(getenv("DFB_GRU_NO48")) : 0;
-    if (use32 && !force && !no48 && B > 15 * 32) return launch_gru_tc_n<48, 256, 1>(s, p);
-    if (use32 && (xg & 2)) return launch_gru_tc_n<32, 256, 1>(s, p);
-    if (!use32 && (xg & 4)) return launch_gru_tc_n<16, 256, 1>(s, p);
-    return use32 ? launch_gru_tc_n<32, 256, 0>(s, p) : launch_gru_tc_n<16, 256, 0>(s, p);
+    if (use32 && B > 15 * 32) return launch_gru_tc_n<48, 256>(s, p);
+    return use32 ? launch_gru_tc_n<32, 256>(s, p) : launch_gru_tc_n<16, 256>(s, p);
 }
 
 int cached_map_f32_sw128(CUtensorMap *out, const void *base, int64_t rows, int64_t cols, int64_t ld, int box_rows);

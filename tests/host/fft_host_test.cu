@@ -1,6 +1,6 @@
 // Host-side emulation of the warp FFT in deepfilternet_b200/csrc/dfb_fft.cuh: runs the 32 lanes
 // sequentially on the CPU and checks against a double-precision DFT.  Built and run by
-// tests/test_fft_host.py (no GPU needed).
+// tests/test_host_logic.py (no GPU needed).
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
