@@ -76,6 +76,8 @@ SIGNATURES = {
     "dfb_features": (_I, [_VP, _VP, _I64, _I64, _I, _F, _VP, _VP, _VP, _VP]),
     "dfb_features_host": (_I, [_VP, _VP, _I64, _I64, _I, _F, _VP, _VP, _VP]),
     "dfb_resample_host": (_I, [_I, _VP, _I64, _I64, _VP, _I, _I, _I, _VP, _I64]),
+    "dfb_metrics": (_I, [_I, _VP, _VP, _VP, _I64, _I64, _I, C.c_uint, _VP, _VP]),
+    "dfb_metrics_host": (_I, [_I, _VP, _VP, _VP, _I64, _I64, _I, C.c_uint, _VP]),
     "dfb_model_create": (_I, [C.POINTER(_VP), _I, C.POINTER(ModelConfigC), C.POINTER(TensorC), _I, _I64P]),
     "dfb_model_free": (None, [_VP]),
     "dfb_model_forward": (_I, [_VP, _VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _VP]),

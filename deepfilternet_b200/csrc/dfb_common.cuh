@@ -195,6 +195,10 @@ bool gl_bx_geometry(int G, int Ig, int Hg, int *gpc_out, int *hgp_out, int *stag
 // DF pathway conv (df_convp) on tensor cores (dfb_tc.cu)
 int launch_df_convp_tc(cudaStream_t s, const float *c0, const float *w_sw, const float *w2, const float *bias, float *coefs, int B, int T,
                        int Fd);
+// torchaudio sinc resampling (dfb_dsp.cu k_resample): x [C][T] -> out [C][T_out] with taps kern [nw][2 width + og] of the
+// gcd-reduced rates; d_lens (device, may be null) gives each row its own length (output ceil(nw lens[c] / og) samples)
+int launch_resample(const float *d_x, int64_t C, int64_t T, const int64_t *d_lens, const float *d_kern, int og, int nw, int width,
+                    float *d_out, int64_t T_out, cudaStream_t s);
 // fp32 [M][K] -> BF16 hi / lo planes [M][K]
 int launch_to_planes(cudaStream_t s, const float *x, int64_t ldx, int64_t M, int K, unsigned short *hi, unsigned short *lo);
 }  // namespace dfb

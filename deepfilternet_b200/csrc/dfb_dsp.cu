@@ -268,8 +268,9 @@ __global__ void k_erb_inv(const float *__restrict__ gains, int64_t n_frames, int
 // enhance.py:56,85): out[c][i * nw + j] = sum_k kern[j][k] * xpad[c][i * og + k], xpad = x zero padded by `width` in
 // front (torchaudio _apply_sinc_resample_kernel: conv1d with stride og).  kern [nw][K = 2 width + og] is built on the
 // host exactly like torchaudio's _get_sinc_resample_kernel (io.py resample_kernel).
-__global__ void __launch_bounds__(256) k_resample(const float *__restrict__ x, int64_t T, const float *__restrict__ kern, int og, int nw,
-                                                  int width, int K, float *__restrict__ out, int64_t Tout) {
+__global__ void __launch_bounds__(256) k_resample(const float *__restrict__ x, int64_t T, const int64_t *__restrict__ lens,
+                                                  const float *__restrict__ kern, int og, int nw, int width, int K,
+                                                  float *__restrict__ out, int64_t Tout) {
     extern __shared__ float s_k[];   // the nw x K taps when they fit (else read through L1)
     const bool in_smem = (size_t)nw * K * sizeof(float) <= 96 * 1024;
     if (in_smem) {
@@ -279,7 +280,10 @@ __global__ void __launch_bounds__(256) k_resample(const float *__restrict__ x, i
     const float *kk = in_smem ? s_k : kern;
     const int c = blockIdx.y;
     const float *xc = x + (int64_t)c * T;
-    for (int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; n < Tout; n += (int64_t)gridDim.x * blockDim.x) {
+    // ragged rows (lens != null): row c holds lens[c] samples (the rest of its T is ignored) and yields
+    // ceil(nw lens[c] / og) outputs, exactly as that row resampled alone
+    const int64_t Tc = lens ? lens[c] : T, Toc = lens ? (nw * Tc + og - 1) / og : Tout;
+    for (int64_t n = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; n < Toc; n += (int64_t)gridDim.x * blockDim.x) {
         const int64_t i = n / nw;
         const int j = (int)(n - i * nw);
         const int64_t p0 = i * og - width;
@@ -287,7 +291,7 @@ __global__ void __launch_bounds__(256) k_resample(const float *__restrict__ x, i
         float acc = 0.f;
         for (int k = 0; k < K; k++) {
             const int64_t p = p0 + k;
-            if (p >= 0 && p < T) acc = fmaf(kr[k], xc[p], acc);
+            if (p >= 0 && p < Tc) acc = fmaf(kr[k], xc[p], acc);
         }
         out[(int64_t)c * Tout + n] = acc;
     }
@@ -762,20 +766,6 @@ __host__ __device__ inline size_t any_warp_bytes(int N, int H, bool syn) {
 }
 __host__ inline size_t any_smem_bytes(int N, int H, int warps, bool syn) {
     return any_cta_bytes(N) + (size_t)warps * any_warp_bytes(N, H, syn);
-}
-
-// inverse / forward M-point transform of buffer a (scratch b) by the warp; returns the buffer holding the result
-template <bool INV>
-__device__ __forceinline__ float2 *warp_fft_any(float2 *a, float2 *b, const float2 *tw, int M, int lane) {
-    for (int r = M, Ns = 1; r > 1;) {
-        const int P = fft_next_radix(r);
-        fft_any_pass<INV>(P, a, b, tw, M, Ns, lane, 32);
-        __syncwarp();
-        Ns *= P;
-        r /= P;
-        float2 *t = a; a = b; b = t;
-    }
-    return a;
 }
 
 // per-CTA tables into shared memory; returns the first per-warp byte
@@ -1447,6 +1437,22 @@ extern "C" int dfb_features_host(dfb_state *st, const float *h_audio, int64_t C,
     return DFB_OK;
 }
 
+namespace dfb {
+int launch_resample(const float *d_x, int64_t C, int64_t T, const int64_t *d_lens, const float *d_kern, int og, int nw, int width,
+                    float *d_out, int64_t T_out, cudaStream_t s) {
+    if (C > 65535) return fail(DFB_ERR_INVALID, "more than 65535 channels per call");
+    const int K = 2 * width + og;
+    const size_t smem = (size_t)nw * K * sizeof(float) <= 96 * 1024 ? (size_t)nw * K * sizeof(float) : 0;
+    static PerDeviceOnce attr_once;
+    if (auto once_guard = attr_once.first()) DFB_CUDA(cudaFuncSetAttribute(k_resample, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+    int64_t blocks = (T_out + 255) / 256;
+    if (blocks > 4096) blocks = 4096;
+    k_resample<<<dim3((unsigned)blocks, (unsigned)C), 256, smem, s>>>(d_x, T, d_lens, d_kern, og, nw, width, K, d_out, T_out);
+    DFB_LAUNCH_CHECK();
+    return DFB_OK;
+}
+}  // namespace dfb
+
 // df/io.py resample (torchaudio.functional.resample): h_audio [C][T] -> h_out [C][T_out]; h_kernel [nw][2 width + og]
 extern "C" int dfb_resample_host(int device, const float *h_audio, int64_t C, int64_t T, const float *h_kernel, int og, int nw,
                                  int width, float *h_out, int64_t T_out) {
@@ -1461,13 +1467,8 @@ extern "C" int dfb_resample_host(int device, const float *h_audio, int64_t C, in
     if (!d_in || !d_out || !d_k) return fail(DFB_ERR_OOM, "cudaMalloc failed");
     DFB_CUDA(cudaMemcpy(d_in, h_audio, sizeof(float) * C * T, cudaMemcpyHostToDevice));
     DFB_CUDA(cudaMemcpy(d_k, h_kernel, sizeof(float) * (size_t)nw * K, cudaMemcpyHostToDevice));
-    const size_t smem = (size_t)nw * K * sizeof(float) <= 96 * 1024 ? (size_t)nw * K * sizeof(float) : 0;
-    static PerDeviceOnce attr_once;
-    if (auto once_guard = attr_once.first()) DFB_CUDA(cudaFuncSetAttribute(k_resample, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
-    int64_t blocks = (T_out + 255) / 256;
-    if (blocks > 4096) blocks = 4096;
-    k_resample<<<dim3((unsigned)blocks, (unsigned)C), 256, smem>>>(d_in, T, d_k, og, nw, width, K, d_out, T_out);
-    DFB_LAUNCH_CHECK();
+    rc = launch_resample(d_in, C, T, nullptr, d_k, og, nw, width, d_out, T_out, 0);
+    if (rc) return rc;
     DFB_CUDA(cudaMemcpy(h_out, d_out, sizeof(float) * C * T_out, cudaMemcpyDeviceToHost));
     return DFB_OK;
 }

@@ -331,4 +331,20 @@ DFB_HD void fft_any_pass(int P, const float2 *src, float2 *dst, const float2 *tw
     }
 }
 
+#ifdef __CUDACC__
+// inverse / forward M-point transform of buffer a (scratch b) by the warp; returns the buffer holding the result
+template <bool INV>
+__device__ __forceinline__ float2 *warp_fft_any(float2 *a, float2 *b, const float2 *tw, int M, int lane) {
+    for (int r = M, Ns = 1; r > 1;) {
+        const int P = fft_next_radix(r);
+        fft_any_pass<INV>(P, a, b, tw, M, Ns, lane, 32);
+        __syncwarp();
+        Ns *= P;
+        r /= P;
+        float2 *t = a; a = b; b = t;
+    }
+    return a;
+}
+#endif
+
 }  // namespace dfb

@@ -121,6 +121,30 @@ int dfb_features_host(dfb_state *st, const float *h_audio, int64_t C, int64_t T,
 int dfb_resample_host(int device, const float *h_audio, int64_t C, int64_t T, const float *h_kernel, int orig, int new_rate,
                       int width, float *h_out, int64_t T_out);
 
+/* ------------------------------------------------------------------ metrics ----------------
+ * Speech-quality metrics of B (clean, degraded) pairs, the device counterpart of the reference's evaluation metrics
+ * (df/stoi.py, df/sepm.py, df/evaluation_utils.py).  One bit per metric; d_out f32[B][popcount(which)] holds the selected
+ * metrics in bit order:
+ *   STOI   df.stoi.stoi at 10 kHz (inputs resampled like df.io.resample); NaN when fewer than 512 samples remain after
+ *          the silent-frame removal (the reference leaves the entry uninitialised)
+ *   SISDR  df.evaluation_utils.si_sdr_speechmetrics at the input rate
+ *   SSNR / LLR / WSS   df.sepm.SNRseg / llr / wss at 16 kHz (inputs resampled to 16 kHz unless sr == 16000, as
+ *          CompositeMetric does); NaN when the 16 kHz signal has fewer than 600 samples (no frame to score) */
+enum {
+    DFB_METRIC_STOI = 1,
+    DFB_METRIC_SISDR = 2,
+    DFB_METRIC_SSNR = 4,
+    DFB_METRIC_LLR = 8,
+    DFB_METRIC_WSS = 16
+};
+/* d_clean / d_deg f32[B][T] (device); lengths: HOST int64[B] (NULL: all T), 1 <= lengths[b] <= T; pair b is scored on its
+ * first lengths[b] samples exactly as if it were scored alone.  sr: 8000, 16000, 22050, 24000, 32000, 44100 or 48000.
+ * Asynchronous on `stream` (device scratch is stream-ordered).  DFB_ERR_INVALID for a bad length, sr or bit. */
+int dfb_metrics(int device, const float *d_clean, const float *d_deg, const int64_t *lengths, int64_t B, int64_t T, int sr,
+                unsigned which, float *d_out, void *stream);
+int dfb_metrics_host(int device, const float *h_clean, const float *h_deg, const int64_t *lengths, int64_t B, int64_t T,
+                     int sr, unsigned which, float *h_out);
+
 /* ------------------------------------------------------------------ model ------------------
  * Replaces the forward pass of DeepFilterNet/df/deepfilternet3.py (DfNet :334-456) and
  * deepfilternet2.py (DfNet :374-505) for the shipped DeepFilterNet2 / 3 / 3_ll topologies. */
